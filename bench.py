@@ -2,6 +2,7 @@
 """bench.py — radar frames/s (ADC cube -> detections) on N B200s, with roofline and CPU baseline.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3|cfg2|cfg4|cfg5|cfg1] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 A step = one pass of the whole chain (range FFT -> Doppler FFT + |X|^2 integration -> 2-D CA-CFAR ->
 detection records incl. angle FFT + grouping -> dense list) over one batch of synthetic frames per GPU.
@@ -19,6 +20,13 @@ Workloads (BASELINE.json configs):
   cfg5  64 sensors x (256 x 128 x 12): latency mode — every frame is its own call; p50/p99 per-frame latency (configs[4])
   cfg1  the reference's own path (100 x 128 x 4, rx0, base-frame subtraction, one 16 384-point FFT, arg-max -> metres)
         through the drop-in library; its CPU baseline is the reference's own code (oracle/_ref, kind "reference") (configs[0])
+--dump-outputs DIR writes what the last timed step returned, one DIR/<name>.npy per array (the inputs are seeded, so two
+builds run with the same arguments can be compared output for output):
+  cfg2/cfg3/cfg4  the ordered detection list of the last batch (rank 0's merged list for N > 1), one array per record field
+  cfg5            the detection lists of the last tick's one-frame calls, one after another, with a sensor column (rank 0's
+                  sensors for N > 1); the device keeps only the last call's list, so the tick is replayed untimed and
+                  read call by call, and its last call is checked against the list the timed loop left
+  cfg1            raw_bin: the arg-max bin of every frame of the last batch (rank 0's for N > 1)
 """
 from __future__ import annotations
 
@@ -162,6 +170,31 @@ def chain_workload_text(name):
     n_theta = 64 if w["A"] <= 64 else 1 << (w["A"] - 1).bit_length()
     return (f"{workload_text(name)}, 2-D CA-CFAR (guard 2x2, train 8x4, alpha 15), {n_theta}-pt angle FFT "
             f"(BASELINE.json configs[{w['idx']}])")
+
+
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy in the narrowest of float32 / float64 that holds it exactly (float32
+    for 16-bit integers and 4-byte floats, float64 otherwise).  All arrays are rows of one table (one entry per detection
+    or frame); past DUMP_BYTES in all, the same fixed, seeded sample of rows is kept from each and its row numbers go to
+    sample_index.npy."""
+    arrays = {k: a.astype(np.float64 if a.dtype.itemsize > 4 or (a.dtype.kind != "f" and a.dtype.itemsize > 2) else np.float32)
+              for k, a in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    keep = (DUMP_BYTES - 1024 * (len(arrays) + 1)) // (sum(a.itemsize for a in arrays.values()) + 8)     # 1 KB per .npy header
+    if n > keep:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["sample_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def detection_fields(dets):
+    return {name: dets[name] for name in dets.dtype.names}
 
 
 def run_reference(args, rank, world):
@@ -318,10 +351,11 @@ STAGE_NAMES = ["range_fft_kernel", "doppler_fft_kernel", "cfar_kernel", "list_ke
 MAX_DET = {"cfg2": 4096, "cfg3": 4096, "cfg4": 32768}
 
 
-def measure_chain(env, name, F, K, W, D, keep_cube=False, e2e_steps=None, share_input=False):
+def measure_chain(env, name, F, K, W, D, keep_cube=False, e2e_steps=None, share_input=False, keep_outputs=False):
     """One chain workload (cfg2 / cfg3 / cfg4) on every rank: K timed steps with D batches in flight (device-resident input,
     CUDA events, max over ranks; for N > 1 each step ends with the exchange of the detection lists), per-stage times of one
-    lane alone, and the end-to-end figure through the host entry points.  Collective: every rank must call it."""
+    lane alone, and the end-to-end figure through the host entry points.  Collective: every rank must call it.
+    keep_outputs: res["last_dets"] is the detection list of the last timed step (rank 0's merged list for N > 1)."""
     torch, pkg, dev, rank, world = env.torch, env.pkg, env.dev, env.rank, env.world
     w = WORKLOADS[name]
     S, C, A, cfg_idx = w["S"], w["C"], w["A"], w["idx"]
@@ -418,6 +452,13 @@ def measure_chain(env, name, F, K, W, D, keep_cube=False, e2e_steps=None, share_
     ms_by_rank = env.all_ranks(ms)
     host_ms_by_rank = env.all_ranks(t_host)
     ms = max(ms_by_rank)
+    last_dets = None
+    if keep_outputs:                                        # before the contexts run anything else
+        last = lanes[(K - 1) % D]
+        if world == 1:
+            last_dets = last.ctx.read_detections()[0]
+        elif rank == 0:
+            last_dets = last.gather.read(pkg.DET_DTYPE)[0]
     frame_counts = ctx.read_counts(F)                       # true per-frame hit counts of this rank's last batch
     hdr = header_view.view(torch.int32).cpu().numpy()
     # the re-FFT detection path (wide arrays in fused mode, or detect_path=2) re-transforms every (frame, range bin) that has
@@ -492,7 +533,7 @@ def measure_chain(env, name, F, K, W, D, keep_cube=False, e2e_steps=None, share_
         exchange=(None if world == 1 else "copy-engine puts into rank 0's memory over NVLink (cudaIpc) + stream wait/write-value flags, one merge kernel on rank 0; "
                   "NCCL for set-up and barriers" if env.exchange == "peer" else "NCCL gather per step + one merge kernel on rank 0"),
         e2e_fps=world * F * e2e_steps / t_e2e, e2e_steps=e2e_steps, e2e_dets=len(dets), e2e_two=len(e2e_ring) > 1,
-        h2d_bytes=F * 4 * N_adc, N_adc=N_adc,
+        h2d_bytes=F * 4 * N_adc, N_adc=N_adc, last_dets=last_dets,
     )
     if world > 1:
         env.sync_all()                                      # no rank unmaps a peer's memory while another may still write to it
@@ -545,7 +586,7 @@ def run_chain(args, env):
     sampler = ClockSampler(env.local_rank)
     if rank == 0:
         sampler.start()
-    res = measure_chain(env, args.workload, F, K, W, D, keep_cube=args.keep_cube)
+    res = measure_chain(env, args.workload, F, K, W, D, keep_cube=args.keep_cube, keep_outputs=bool(args.dump_outputs))
     # the other BASELINE.json configs beside the headline shape, on the same box and the same N: configs[1] (cfg2),
     # configs[3] (cfg4, frame-sharded) and configs[4] (cfg5, sensors sharded) — shorter runs, same method
     others = {}
@@ -618,13 +659,16 @@ def run_chain(args, env):
             line["cpu_baseline"] = {"value": n / dt, "unit": "frames/s", "cores": port.cores, "kind": "port",
                                     "sample": f"{n} frames ({port.pool.shape[0]} distinct, {passes} passes) of the same workload in {dt:.1f} s; "
                                               f"plain-C fp64 oracle (the reference has no CPU code for these stages), {port.cores} OpenMP threads"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, detection_fields(res["last_dets"]))
         env.emit(line)
 
 
-def measure_stream(env, name, sensors_total, K, W, depth=4, graph=True):
+def measure_stream(env, name, sensors_total, K, W, depth=4, graph=True, keep_outputs=False):
     """cfg5: 64 sensors x (256 x 128 x 12) at 30 fps — latency mode.  Every frame is its own call (a sensor's frame is
     processed the moment it arrives); sensors are pinned to GPUs (sensor mod N).  A step = one tick = one frame from
-    every sensor of this rank.  Collective: every rank must call it."""
+    every sensor of this rank.  Collective: every rank must call it.
+    keep_outputs: res["last_tick"] holds the detection lists of the last device-resident tick, with a sensor column."""
     torch, pkg, dev, rank, world = env.torch, env.pkg, env.dev, env.rank, env.world
     w = WORKLOADS[name]
     S, C, A, cfg_idx = w["S"], w["C"], w["A"], w["idx"]
@@ -673,6 +717,17 @@ def measure_stream(env, name, sensors_total, K, W, depth=4, graph=True):
     e1.record(st)
     env.sync_all()
     ms = env.max_over_ranks(e0.elapsed_time(e1))
+    last_tick = None
+    if keep_outputs:
+        # the device holds only the last call's list: the last tick is replayed untimed (same inputs, context and frame
+        # offset) and read call by call; its last call must give back the list the timed loop left behind
+        timed_last = ctx.read_detections()[0]
+        lists = []
+        for i in range(F):
+            ctx.process_device(dframes[i], 1)
+            lists.append(ctx.read_detections()[0])
+        assert lists[-1].tobytes() == timed_last.tobytes(), "cfg5: the replayed tick differs from the timed one"
+        last_tick = dict(detection_fields(np.concatenate(lists)), sensor=np.repeat(np.array(sensors), [len(d) for d in lists]))
 
     # host path: every frame H2D -> chain -> D2H, synchronous per frame; wall-clock latency per call
     for _ in range(W):
@@ -730,7 +785,7 @@ def measure_stream(env, name, sensors_total, K, W, depth=4, graph=True):
         kernels_per_batch=int(ctx.info.kernels_per_batch), frame_shorts=ctx.frame_shorts,
         lat_p50=float(lat_us[len(lat_us) // 2]), lat_p99=float(lat_us[min(len(lat_us) - 1, int(0.99 * len(lat_us)))]),
         lat_max=float(lat_us[-1]), lat_n=int(len(lat_us)), tick_batched_ms=tick_batched_ms,
-        sync_fps=sensors_total * K / t_sync, pipe_fps=sensors_total * K / t_pipe, t_pipe=t_pipe, n_det=n_det,
+        sync_fps=sensors_total * K / t_sync, pipe_fps=sensors_total * K / t_pipe, t_pipe=t_pipe, n_det=n_det, last_tick=last_tick,
     )
     ctx.close()
     del adc, host
@@ -765,7 +820,8 @@ def run_stream(args, env):
     sampler = ClockSampler(env.local_rank)
     if rank == 0:
         sampler.start()
-    res = measure_stream(env, args.workload, sensors_total, K, W, depth=args.depth, graph=not args.no_graph)
+    res = measure_stream(env, args.workload, sensors_total, K, W, depth=args.depth, graph=not args.no_graph,
+                         keep_outputs=bool(args.dump_outputs))
     clocks = sampler.stop() if rank == 0 else None
     F, ms = res["F"], res["ms"]
     if rank == 0:
@@ -804,6 +860,8 @@ def run_stream(args, env):
             n, dt, _ = port.run(port.passes_for(12.0))
             line["cpu_baseline"] = {"value": n / dt, "unit": "frames/s", "cores": port.cores, "kind": "port",
                                     "sample": f"{n} frames in {dt:.1f} s, plain-C fp64 oracle, {port.cores} OpenMP threads (frame-parallel)"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, res["last_tick"])
         env.emit(line)
 
 
@@ -883,6 +941,8 @@ def run_legacy(args, env):
             line["cpu_baseline"] = {"value": n / dt, "unit": "frames/s", "cores": 1, "kind": port.kind,
                                     "sample": f"{n} frames in {dt:.1f} s through the reference's cpuTiming() loop body "
                                               f"({'compiled from /root/reference into oracle/_ref' if port.kind == 'reference' else 'oracle restatement'}), single thread like the reference"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"raw_bin": got})
         env.emit(line)
 
 
@@ -903,7 +963,13 @@ def main():
     ap.add_argument("--depth", type=int, default=4, help="cfg5: one-frame calls in flight on the end-to-end path (ring of contexts, mmw_submit_host / mmw_wait)")
     ap.add_argument("--no-graph", action="store_true", help="cfg5: launch the kernels one by one instead of replaying a CUDA graph")
     ap.add_argument("--keep-cube", action="store_true", help="materialise the Doppler cube in HBM (default: fused)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (the detection list field by field; cfg1: the arg-max bins) "
+                                                             "as DIR/<name>.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.impl == "reference":

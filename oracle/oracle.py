@@ -272,6 +272,32 @@ def ref_cpu_frame(frame: np.ndarray, base_rx0: np.ndarray, want_spectrum=False):
     return (d, raw.value, spec) if want_spectrum else (d, raw.value)
 
 
+# the comparison of tests/test_oracle_pin.py::test_against_compiled_reference as arrays: computed with the reference's
+# functions it is what tests/golden/make_golden.py stores (legacy_reference_direct.npz), with the oracle's what is compared
+DIRECT_FFT_SIZES = (2, 16, 4096, 16384)
+DIRECT_POW2_ARGS = (1, 2, 3, 100, 12800, 16384, 16385)
+DIRECT_BINS = np.sort(np.random.default_rng(11).choice(16384, 2048, replace=False))   # stored sample of 16384-point outputs
+
+
+def direct_vectors(cap, reshape, cpu_frame, fft, next_pow2, sample=False):
+    """cap: legacy capture, frame 0 the base frame.  reshape / cpu_frame / fft / next_pow2: the reference's functions
+    (ref_*) or the oracle's.  sample: keep only DIRECT_BINS of the 16384-point spectra and FFT."""
+    pick = (lambda a: a[DIRECT_BINS]) if sample else (lambda a: a)
+    y = reshape(cap[0])
+    out = {"reshape0": y, "pow2": np.array([next_pow2(n) for n in DIRECT_POW2_ARGS])}
+    dist, raw = [], []
+    for f in range(1, cap.shape[0]):
+        d, r, spec = cpu_frame(cap[f], y[:12800], want_spectrum=True)
+        dist.append(d)
+        raw.append(r)
+        out[f"spec{f}"] = pick(spec)
+    out["dist"], out["raw"] = np.array(dist), np.array(raw)
+    for n in DIRECT_FFT_SIZES:
+        X = fft(np.random.default_rng(n).normal(size=n) + 0j)
+        out[f"fft{n}"] = pick(X) if n == 16384 else X
+    return out
+
+
 def ref_cpu_time_frames(frames: np.ndarray, base_rx0: np.ndarray):
     """Seconds the reference CPU loop body takes for frames[n][102400] on one thread."""
     frames = np.ascontiguousarray(frames, np.int16)

@@ -1,11 +1,12 @@
-"""Generates tests/golden/legacy_reference.npz from the REFERENCE's own CPU functions.
+"""Generates tests/golden/legacy_reference.npz and legacy_reference_direct.npz from the REFERENCE's
+own CPU functions.
 
-Run in the build container (needs /root/reference):  python tests/golden/make_golden.py
+Run where the reference's sources are (oracle/Makefile, REF):  python tests/golden/make_golden.py
 It calls the reference code compiled by oracle/Makefile into oracle/_ref/libref_cpu.so
 (ReshapeComplex_t, butterfly_fft, FindAbsMax and the cpuTiming() loop body,
 cudaBenchMarking.cpp:61-105, :149-206, :273-303) on seeded synthetic captures in the
-fhy_direct.bin format and stores the outputs.  The GPU box has no /root/reference: the tests
-there read only this file.
+fhy_direct.bin format and stores the outputs.  A checkout without those sources tests against
+these files alone.
 """
 import os
 import sys
@@ -59,4 +60,10 @@ for n in (64, 128, 256, 512, 1024):
     out[f"fft{n}_out"] = orc.ref_fft(x)
 path = os.path.join(ROOT, "tests", "golden", "legacy_reference.npz")
 np.savez_compressed(path, **out)
+print("wrote", path, os.path.getsize(path), "bytes")
+# (5) the direct comparison of tests/test_oracle_pin.py::test_against_compiled_reference, for checkouts without oracle/_ref
+direct = orc.direct_vectors(pkg.synth.legacy_capture(4, seed=11), orc.ref_reshape, orc.ref_cpu_frame, orc.ref_fft,
+                            orc.ref().ref_next_pow2, sample=True)
+path = os.path.join(ROOT, "tests", "golden", "legacy_reference_direct.npz")
+np.savez_compressed(path, **direct)
 print("wrote", path, os.path.getsize(path), "bytes")
