@@ -38,7 +38,7 @@ C_ABI_SYMBOLS = [
     "mmw_set_windows", "mmw_get_windows", "mmw_set_frame_offset", "mmw_stream", "mmw_use_stream",
     "mmw_process_device", "mmw_process_host", "mmw_submit_host", "mmw_wait", "mmw_read_detections", "mmw_read_counts",
     "mmw_device_results", "mmw_device_result_block", "mmw_merge_gathered", "mmw_copy_range_spectrum", "mmw_copy_doppler_cube", "mmw_copy_power_map",
-    "mmw_copy_cfar_mask", "mmw_time_device", "mmw_front_stats", "mmw_check_guards", "mmw_set_detect_path",
+    "mmw_copy_cfar_mask", "mmw_time_device", "mmw_check_guards", "mmw_set_detect_path",
     "mmw_set_graph_mode", "mmw_set_base_frame", "mmw_process_capture_file", "mmw_default_radar_params", "mmw_to_physical",
     "mmw_legacy_process_frame", "mmw_legacy_process_frames", "mmw_legacy_copy_spectrum", "mmw_legacy_shutdown",
     "mmw_legacy_process_device", "mmw_legacy_sync", "mmw_legacy_distance_from_raw", "mmw_legacy_process_file",
@@ -129,7 +129,6 @@ def load(build_if_missing: bool = True):
     for name in ("mmw_copy_range_spectrum", "mmw_copy_doppler_cube", "mmw_copy_power_map", "mmw_copy_cfar_mask"):
         getattr(L, name).argtypes = [vp, C.c_int, vp]
     L.mmw_time_device.argtypes = [vp, vp, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float)]
-    L.mmw_front_stats.argtypes = [vp, vp, C.c_int]
     L.mmw_check_guards.argtypes = [vp, C.POINTER(C.c_longlong)]
     L.mmw_set_detect_path.argtypes = [vp, C.c_int]
     L.mmw_exchange_create.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(vp)]
@@ -421,14 +420,6 @@ class RadarContext:
         bad = C.c_longlong(0)
         _check(self._L.mmw_check_guards(self._h, C.byref(bad)))
         return int(bad.value)
-
-    def front_stats(self, max_ctas: int = 1024) -> np.ndarray:
-        """Per-CTA record of the last fused-front launch (MMW_FRONT_STATS=1 at create): [n, 8] uint64."""
-        out = np.zeros((max_ctas, 8), dtype=np.uint64)
-        n = self._L.mmw_front_stats(self._h, _np_ptr(out), max_ctas)
-        if n < 0:
-            _check(n)
-        return out[:n]
 
 
 class PeerExchange:

@@ -17,7 +17,6 @@ SOURCES = ["mmw_api.cu", "mmw_pipeline.cu", "mmw_detect.cu", "mmw_legacy.cu"]
 HEADERS = [
     os.path.join(CSRC, "fft_regs.cuh"),
     os.path.join(CSRC, "mmw_common.cuh"),
-    os.path.join(CSRC, "mmw_front.cuh"),
     os.path.join(ROOT, "include", "mmw_radar.h"),
     os.path.join(ROOT, "include", "mmw_legacy.h"),
 ]

@@ -40,7 +40,6 @@ static int next_pow2(int n)
 using namespace mmw;
 
 constexpr int kMaxChunks = 32;
-constexpr int kFrontStatsCtas = 1024;     // CTAs the optional timing record of the fused front kernel has room for
 constexpr int kResultHeaderBytes = MMW_RESULT_HEADER_BYTES;
 
 struct mmw_ctx {
@@ -68,9 +67,7 @@ struct mmw_ctx {
     uint32_t *d_counts;
     uint32_t *d_offsets;
     unsigned int *d_ticket;
-    unsigned long long *d_front_stats;   // MMW_FRONT_STATS=1 only
     unsigned int *d_sched;        // PlanDev.sched
-    unsigned int *d_front_sync;   // produced / consumed slab counters of the fused front kernel, [2][max_frames * A]
     uint4 *d_rows;            // hit rows of the selective Doppler re-FFT (wide arrays, fused mode)
     float2 *d_snap;           // antenna snapshots of the detected cells (same path)
     unsigned char *d_result;  // [32-byte header | dense ordered detection list]: one D2H usually moves both
@@ -240,8 +237,8 @@ void mmw_destroy(mmw_ctx *c)
     if (!c) return;
     cudaSetDevice(c->device);
     void *bufs[] = {c->d_win_r, c->d_win_d, c->d_tw1_r, c->d_tw1_d, c->d_tw_d, c->d_tw_a, c->d_adc, c->d_base, c->d_rs, c->d_cube, c->d_pmap,
-                    c->d_psplit, c->d_mask, c->d_noise, c->d_keys, c->d_counts, c->d_offsets, c->d_ticket, c->d_front_sync, c->d_sched,
-                    c->d_front_stats, c->d_rows, c->d_snap, c->d_result};
+                    c->d_psplit, c->d_mask, c->d_noise, c->d_keys, c->d_counts, c->d_offsets, c->d_ticket, c->d_sched,
+                    c->d_rows, c->d_snap, c->d_result};
     for (void *b : bufs) dev_free(c, b);
     cudaFree(c->d_scratch);
     delete c->guards;
@@ -338,15 +335,14 @@ int mmw_create(const mmw_config *cfg, mmw_ctx **out)
     if ((rc = dev_alloc(c, &c->d_counts, (size_t)F))) return fail(rc);
     if ((rc = dev_alloc(c, &c->d_offsets, (size_t)F + 1))) return fail(rc);
     if ((rc = dev_alloc(c, &c->d_ticket, (size_t)4))) return fail(rc);
-    if ((rc = dev_alloc(c, &c->d_front_sync, (size_t)2 * F * A))) return fail(rc);
     if ((rc = dev_alloc(c, &c->d_sched, (size_t)8))) return fail(rc);
     if (cudaMemset(c->d_sched, 0, 8 * sizeof(unsigned int)) != cudaSuccess) { set_last_error("cudaMemset failed"); return fail(MMW_ERR_CUDA); }
     if (cudaMemset(c->d_ticket, 0, 4 * sizeof(unsigned int)) != cudaSuccess) { set_last_error("cudaMemset failed"); return fail(MMW_ERR_CUDA); }
     c->dense_cap = F * cfg->max_det_per_frame;
     // wide arrays without a Doppler cube: snapshots of the detected cells come from a selective re-FFT of the hit rows
     // (launch_detect); its buffers scale with the detection capacity — beyond 2 GB the per-detection kernel is used instead.
-    // Narrow arrays get them when the caller picks that path (mmw_set_detect_path, or MMW_K4_VARIANT=2 in the environment).
-    if ((A >= 32 || env_int("MMW_K4_VARIANT") == 2) && (rc = alloc_refft_buffers(c))) return fail(rc);
+    // Narrow arrays get them when the caller picks that path (mmw_set_detect_path).
+    if (A >= 32 && (rc = alloc_refft_buffers(c))) return fail(rc);
     const size_t result_bytes = kResultHeaderBytes + (size_t)c->dense_cap * sizeof(mmw_detection);
     if ((rc = dev_alloc(c, &c->d_result, result_bytes))) return fail(rc);
     c->d_header = reinterpret_cast<uint32_t *>(c->d_result);
@@ -379,18 +375,8 @@ int mmw_create(const mmw_config *cfg, mmw_ctx **out)
     p.max_det = cfg->max_det_per_frame; p.keep_cube = cfg->keep_doppler_cube ? 1 : 0; p.frame_offset = 0;
     p.base_adc = nullptr;
     p.sched = c->d_sched;
-    // kernel-shape overrides of the sweeps under profiles/ and of the kernel-form parity tests: read once, here
-    p.k1_variant = env_int("MMW_K1_VARIANT"); p.k2_variant = env_int("MMW_K2_VARIANT"); p.k3_variant = env_int("MMW_K3_VARIANT");
-    p.k4_variant = env_int("MMW_K4_VARIANT"); p.ctas_per_sm_cap = env_int("MMW_CTAS_PER_SM");
-    p.front_variant = env_int("MMW_FRONT"); p.front_window = env_int("MMW_FRONT_WINDOW");
-    p.reserve_ctas = env_int("MMW_RESERVE_CTAS");
+    p.detect_path = MMW_DETECT_AUTO;
     p.sched_dynamic = getenv("MMW_SCHED") ? env_int("MMW_SCHED") : 1;
-    p.front_stats = nullptr;
-    if (env_int("MMW_FRONT_STATS")) {
-        if ((rc = dev_alloc(c, &c->d_front_stats, (size_t)kFrontStatsCtas * 8))) return fail(rc);
-        if (cudaMemset(c->d_front_stats, 0, (size_t)kFrontStatsCtas * 8 * sizeof(unsigned long long)) != cudaSuccess) { set_last_error("cudaMemset failed"); return fail(MMW_ERR_CUDA); }
-        p.front_stats = c->d_front_stats;
-    }
     p.win_r = c->d_win_r; p.win_d = c->d_win_d; p.tw_d = c->d_tw_d; p.tw_a = c->d_tw_a; p.tw1_r = c->d_tw1_r; p.tw1_d = c->d_tw1_d;
 
     // antenna-split Doppler path of small batches (run_front): per-antenna power maps for the largest batch that still
@@ -418,7 +404,8 @@ int mmw_get_info(const mmw_ctx *c, mmw_info *info)
     info->algorithmic_bytes_per_frame = 28 * N + 8 * M;
     info->workspace_bytes = (long long)c->workspace_bytes;
     // K1, K2, K3, list, measure; the selective re-FFT path runs rows + extract + angle instead of measure (launch_detect's rule)
-    info->kernels_per_batch = ((p.A >= 32 || p.k4_variant == 2) && !p.keep_cube && c->d_snap != nullptr && p.k4_variant != 1) ? 7 : 5;
+    info->kernels_per_batch = ((p.A >= 32 || p.detect_path == MMW_DETECT_REFFT) && !p.keep_cube && c->d_snap != nullptr &&
+                               p.detect_path != MMW_DETECT_PER_CELL) ? 7 : 5;
     return MMW_OK;
 }
 
@@ -487,11 +474,11 @@ int mmw_set_detect_path(mmw_ctx *c, int path)
         int rc = alloc_refft_buffers(c);
         if (rc) return rc;
     }
-    if (c->plan.k4_variant != path && c->graphs) {      // the captured launch sequences belong to the old path
+    if (c->plan.detect_path != path && c->graphs) {     // the captured launch sequences belong to the old path
         CK(cudaStreamSynchronize(c->stream));
         destroy_graphs(c);
     }
-    c->plan.k4_variant = path;                           // 0 / 1 / 2: the launcher's own numbering (launch_detect)
+    c->plan.detect_path = path;
     return MMW_OK;
 }
 
@@ -502,13 +489,6 @@ int mmw_use_stream(mmw_ctx *c, void *cuda_stream)
     if (!c) { set_last_error("mmw_use_stream: null context"); return MMW_ERR_ARG; }
     c->stream = cuda_stream ? (cudaStream_t)cuda_stream : c->own_stream;
     return MMW_OK;
-}
-
-static bool front_uses_fused(const PlanDev &p, int n_frames)
-{
-    if (p.front_variant == 1) return false;
-    if (p.front_variant != 2 && p.front_variant != 3) return false;  // default: two kernels (until measured otherwise)
-    return front_fused_supported(p, n_frames);
 }
 
 // stages 1-3 on frames [first, first + n) of the batch (they are per-frame independent)
@@ -522,15 +502,6 @@ static int run_front(mmw_ctx *c, const int16_t *adc_dev, int first, int n, cudaE
     float2 *cube = p.keep_cube ? c->d_cube + (size_t)first * p.A * M : nullptr;
     if (stage_ev) CK(cudaEventRecord(stage_ev[0], st));
     const bool split = !cube && n <= c->psplit_frames && doppler_prefers_split(p, n);     // d_psplit: mmw_create
-    if (!split && front_uses_fused(p, n)) {
-        // K1 and K2 as the two roles of one kernel: the Doppler role reads the range spectrum out of the L2 (mmw_front.cuh)
-        CK(launch_front_fused(p, adc, rs, c->d_pmap + (size_t)first * M, n, c->d_front_sync, st));
-        if (stage_ev) CK(cudaEventRecord(stage_ev[1], st));          // (no boundary between the two stages: all of it is booked on stage 1)
-        if (stage_ev) CK(cudaEventRecord(stage_ev[2], st));
-        CK(launch_cfar(p, c->d_pmap + (size_t)first * M, c->d_mask + (size_t)first * (M / 32), c->d_noise + (size_t)first * M, n, c->sm_count, st));
-        if (stage_ev) CK(cudaEventRecord(stage_ev[3], st));
-        return MMW_OK;
-    }
     CK(launch_range_fft(p, adc, rs, n, st));
     if (stage_ev) CK(cudaEventRecord(stage_ev[1], st));
     if (split) {
@@ -1206,17 +1177,6 @@ int mmw_copy_cfar_mask(mmw_ctx *c, int frame, uint8_t *out)
     CK(cudaStreamSynchronize(c->stream));
     CK(cudaMemcpy(out, c->d_scratch, n, cudaMemcpyDeviceToHost));
     return MMW_OK;
-}
-
-int mmw_front_stats(mmw_ctx *c, unsigned long long *out, int max_ctas)
-{
-    if (!c || !out || max_ctas < 1) { set_last_error("mmw_front_stats: bad argument"); return MMW_ERR_ARG; }
-    if (!c->d_front_stats) { set_last_error("mmw_front_stats: the context was created without MMW_FRONT_STATS=1"); return MMW_ERR_STATE; }
-    CK(cudaSetDevice(c->device));
-    CK(cudaStreamSynchronize(c->stream));
-    const int n = max_ctas < kFrontStatsCtas ? max_ctas : kFrontStatsCtas;
-    CK(cudaMemcpy(out, c->d_front_stats, (size_t)n * 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-    return n;
 }
 
 int mmw_check_guards(mmw_ctx *c, long long *bad_bytes)

@@ -28,16 +28,14 @@ struct PlanDev {
     const float2 *tw_a;     // [n_theta]
     unsigned int *sched;    // [8] work counters of the persistent FFT kernels: {next item, CTAs retired} for K1 at [0], K2 at [2]; zero between launches
     const int16_t *base_adc; // one frame [C][A][S] IIQQ subtracted before the range window, or nullptr (static-clutter removal)
-    // host-side only: kernel-shape overrides for the sweeps under profiles/ and the kernel-form parity tests.  Read ONCE, in
-    // mmw_create (MMW_K1_VARIANT / MMW_K2_VARIANT / MMW_K3_VARIANT / MMW_K4_VARIANT / MMW_CTAS_PER_SM); 0 = pick by shape.
-    int k1_variant, k2_variant, k3_variant, k4_variant, ctas_per_sm_cap;
+    int detect_path;        // host-side only: MMW_DETECT_AUTO / _PER_CELL / _REFFT (mmw_set_detect_path), read by launch_detect
     int sched_dynamic;      // bit 0: K1, bit 1: K2 take their tiles from PlanDev.sched instead of a fixed stride (MMW_SCHED; default 1)
-    int reserve_ctas;       // CTA slots the persistent FFT kernels leave free for kernels of other streams (mmw_reserve_ctas; MMW_RESERVE_CTAS)
-    // MMW_FRONT: 0 = pick (fused front where supported), 1 = K1 and K2 as two kernels, 2 = fused front wherever supported;
-    // MMW_FRONT_WINDOW: slabs the producer role may run ahead of the consumer role (0 = derived from the grid)
-    int front_variant, front_window;
-    unsigned long long *front_stats;   // MMW_FRONT_STATS=1: per-CTA timing record of the fused front kernel (mmw_front_stats), else nullptr
+    // Padding to a multiple of 16 bytes: the pointer arguments after the plan then keep their 16-byte pairing, which the
+    // compiler loads with one 128-bit constant load (measure_wide_kernel).  alignas(16) would do the same but changes
+    // the code of the kernels that read the plan's first fields.
+    int pad_[2];
 };
+static_assert(sizeof(PlanDev) % 16 == 0, "PlanDev size");
 
 // internal HBM layouts (DESIGN.md §3)
 //   adc   [F][C][A][S]  int16 IIQQ   (the reference's capture format)
@@ -103,10 +101,6 @@ __device__ __forceinline__ void st_global_f2(float2 *p, float2 v)
 // ---------------------------------------------------------------------------
 cudaError_t launch_range_fft(const PlanDev &p, const int16_t *adc, float2 *rs, int n_frames, cudaStream_t st);
 cudaError_t launch_doppler_fft(const PlanDev &p, const float2 *rs, float2 *cube, float *pmap, int n_frames, cudaStream_t st);
-// K1 + K2 as one cooperative kernel whose Doppler role reads the range spectrum back out of the L2 (mmw_front.cuh);
-// sync: 2 * n_frames * A counters (zeroed by the launcher)
-bool front_fused_supported(const PlanDev &p, int n_frames);
-cudaError_t launch_front_fused(const PlanDev &p, const int16_t *adc, float2 *rs, float *pmap, int n_frames, unsigned int *sync, cudaStream_t st);
 // small batches: K2 over F*A single-antenna frames into per-antenna maps, then the ordered sum (mmw_pipeline.cu)
 bool doppler_prefers_split(const PlanDev &p, int n_frames);
 cudaError_t launch_power_sum(const PlanDev &p, const float *per_antenna, float *pmap, int n_frames, cudaStream_t st);

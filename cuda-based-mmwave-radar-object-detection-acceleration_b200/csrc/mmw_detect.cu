@@ -35,25 +35,16 @@ constexpr int kCfarDT = 32;      // Doppler bins per tile (one mask word per ran
 constexpr int kCfarNT = 256;
 constexpr int kCfarRS = kCfarRT + 4;   // row stride of the row-sum arrays (16-byte aligned rows)
 
-// FIXED = the default geometry (guard 2x2, train 8x4): fully unrolled register-window version.
-// Generic geometries take the run-time-bound version below (same sums, same association per cell).
-//
-// FIXED data flow per 64 x 32 tile (+ halo 10 range / 6 Doppler):
-//   load   tile[44][84]                              coalesced, Doppler wrapped, range zero-filled
-//   rows   a thread makes 8 adjacent range cells of one row from 28 register values: sliding sums by
-//          pairwise doubling (s2 -> s4 -> s8), no subtraction anywhere
-//   cols   a thread makes 4 adjacent Doppler cells of one range bin from 22 register values (lanes run
-//          along range, so every shared-memory access is stride-1)
-//   hits   4 bits per thread OR-ed into the tile's 64 mask words; noise stored for hit cells only
-template <bool FIXED>
+// Tiled CFAR for any guard / training window other than the default one (that one takes cfar_walk_kernel below):
+// one CTA per 64 x 32 tile plus its halo, run-time window bounds, one cell at a time.
 __global__ void __launch_bounds__(kCfarNT) cfar_kernel(PlanDev p, const float *__restrict__ pmap, uint32_t *__restrict__ mask,
                                                        float *__restrict__ noise_map)
 {
     extern __shared__ __align__(16) unsigned char smem[];
-    const int Gr = FIXED ? 2 : p.guard_r, Gd = FIXED ? 2 : p.guard_d;
-    const int Wr = FIXED ? 10 : p.win_r_half, Wd = FIXED ? 6 : p.win_d_half;
+    const int Gr = p.guard_r, Gd = p.guard_d;
+    const int Wr = p.win_r_half, Wd = p.win_d_half;
     const int Sp = p.Sp, Cp = p.Cp;
-    const int Lp = FIXED ? 12 : ((Wr + 3) & ~3);         // halo rounded up to whole float4 chunks
+    const int Lp = (Wr + 3) & ~3;                        // halo rounded up to whole float4 chunks
     const int tw_ = kCfarRT + 2 * Lp;                    // tile width (range, fastest)
     const int th_ = kCfarDT + 2 * Wd;                    // tile height (Doppler)
     constexpr int RS = kCfarRS;
@@ -88,107 +79,33 @@ __global__ void __launch_bounds__(kCfarNT) cfar_kernel(PlanDev p, const float *_
     }
     __syncthreads();
 
-    if constexpr (FIXED) {
-        // ---- row pass: 44 rows x 8 segments of 8 cells ----
-        for (int t = tid; t < 44 * (kCfarRT / 8); t += kCfarNT) {
-            const int j = t >> 3, x0 = (t & 7) * 8;
-            const float4 *c4 = reinterpret_cast<const float4 *>(tile + j * tw_ + x0);   // v[i] = offset (i - 12) of cell x0
-            float v[32];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const float4 q = c4[i];
-                v[4 * i] = q.x; v[4 * i + 1] = q.y; v[4 * i + 2] = q.z; v[4 * i + 3] = q.w;
-            }
-            float s2[31], s4[29], ring[8], full[8];
-#pragma unroll
-            for (int i = 0; i < 31; ++i) s2[i] = v[i] + v[i + 1];
-#pragma unroll
-            for (int i = 0; i < 29; ++i) s4[i] = s2[i] + s2[i + 2];
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                const float left = s4[q + 2] + s4[q + 6];         // v[q+2 .. q+9]    offsets -10 .. -3
-                const float right = s4[q + 15] + s4[q + 19];      // v[q+15 .. q+22]  offsets  +3 .. +10
-                const float mid = s4[q + 10] + v[q + 14];         // v[q+10 .. q+14]  offsets  -2 .. +2
-                ring[q] = left + right;
-                full[q] = ring[q] + mid;
-            }
-            float4 *fo = reinterpret_cast<float4 *>(fullS + j * RS + x0);
-            float4 *ro = reinterpret_cast<float4 *>(ringS + j * RS + x0);
-            fo[0] = make_float4(full[0], full[1], full[2], full[3]);
-            fo[1] = make_float4(full[4], full[5], full[6], full[7]);
-            ro[0] = make_float4(ring[0], ring[1], ring[2], ring[3]);
-            ro[1] = make_float4(ring[4], ring[5], ring[6], ring[7]);
+    for (int t = tid; t < th_ * kCfarRT; t += kCfarNT) {
+        const int j = t / kCfarRT, x = t % kCfarRT;
+        const float *c = tile + j * tw_ + x + (Lp - Wr);   // c[i] = offset (i - Wr)
+        float left = 0.f, right = 0.f, mid = 0.f;
+        for (int i = 0; i < Wr - Gr; ++i) left += c[i];
+        for (int i = Wr + Gr + 1; i <= 2 * Wr; ++i) right += c[i];
+        for (int i = Wr - Gr; i <= Wr + Gr; ++i) mid += c[i];
+        ringS[j * RS + x] = left + right;
+        fullS[j * RS + x] = (left + right) + mid;
+    }
+    __syncthreads();
+    for (int t = tid; t < kCfarDT * kCfarRT; t += kCfarNT) {
+        const int x = t % kCfarRT, dl = t / kCfarRT;
+        const int r = r0 + x;
+        float T = 0.f;
+        for (int jj = 0; jj <= 2 * Wd; ++jj) {
+            const float *src = (jj >= Wd - Gd && jj <= Wd + Gd) ? ringS : fullS;
+            T += src[(dl + jj) * RS + x];
         }
-        __syncthreads();
-
-        // ---- column pass: 64 range bins x 8 groups of 4 Doppler cells; lanes along range ----
-#pragma unroll
-        for (int it = 0; it < 2; ++it) {
-            const int t = tid + it * kCfarNT;
-            const int x = t & 63, g = t >> 6;              // range bin in tile, Doppler group
-            const int r = r0 + x;
-            const float *fc = fullS + (4 * g) * RS + x;    // row index = Doppler offset + 6 relative to d0 + 4 g
-            const float *rc = ringS + (4 * g) * RS + x;
-            float fu[16], rg[8];
-#pragma unroll
-            for (int i = 0; i < 16; ++i) fu[i] = (i < 7 || i > 8) ? fc[i * RS] : 0.f;   // full rows 0..6, 9..15
-#pragma unroll
-            for (int i = 0; i < 8; ++i) rg[i] = rc[(i + 4) * RS];                       // ring rows 4..11
-            float f2[15], r2[7];
-#pragma unroll
-            for (int i = 0; i < 15; ++i) f2[i] = fu[i] + fu[i + 1];
-#pragma unroll
-            for (int i = 0; i < 7; ++i) r2[i] = rg[i] + rg[i + 1];
-            const int n_full = min(r + 10, Sp - 1) - max(r - 10, 0) + 1;
-            const int n_guard = min(r + 2, Sp - 1) - max(r - 2, 0) + 1;
-            const int n = 13 * n_full - 5 * n_guard;
-            const float inv_n = 1.0f / (float)n;
-            uint32_t bits = 0;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const float top = f2[q] + f2[q + 2];                   // full rows q .. q+3      (Doppler offsets -6 .. -3)
-                const float bot = f2[q + 9] + f2[q + 11];              // full rows q+9 .. q+12   (offsets +3 .. +6)
-                const float gd = (r2[q] + r2[q + 2]) + rg[q + 4];      // ring rows q+4 .. q+8    (offsets -2 .. +2)
-                const float noise = ((top + bot) + gd) * inv_n;
-                const float cut = tile[(4 * g + q + 6) * tw_ + x + 12];
-                const bool hit = (r < Sp) && (cut > p.alpha * noise);
-                if (hit) {
-                    bits |= 1u << (4 * g + q);
-                    noise_map[((size_t)f * Cp + d0 + 4 * g + q) * Sp + r] = noise;      // sparse: hit cells only
-                }
-            }
-            if (bits) atomicOr(&words[x], bits);
-        }
-    } else {
-        // ---- generic geometry: run-time bounds, one cell at a time ----
-        for (int t = tid; t < th_ * kCfarRT; t += kCfarNT) {
-            const int j = t / kCfarRT, x = t % kCfarRT;
-            const float *c = tile + j * tw_ + x + (Lp - Wr);   // c[i] = offset (i - Wr)
-            float left = 0.f, right = 0.f, mid = 0.f;
-            for (int i = 0; i < Wr - Gr; ++i) left += c[i];
-            for (int i = Wr + Gr + 1; i <= 2 * Wr; ++i) right += c[i];
-            for (int i = Wr - Gr; i <= Wr + Gr; ++i) mid += c[i];
-            ringS[j * RS + x] = left + right;
-            fullS[j * RS + x] = (left + right) + mid;
-        }
-        __syncthreads();
-        for (int t = tid; t < kCfarDT * kCfarRT; t += kCfarNT) {
-            const int x = t % kCfarRT, dl = t / kCfarRT;
-            const int r = r0 + x;
-            float T = 0.f;
-            for (int jj = 0; jj <= 2 * Wd; ++jj) {
-                const float *src = (jj >= Wd - Gd && jj <= Wd + Gd) ? ringS : fullS;
-                T += src[(dl + jj) * RS + x];
-            }
-            const int n_full = min(r + Wr, Sp - 1) - max(r - Wr, 0) + 1;
-            const int n_guard = min(r + Gr, Sp - 1) - max(r - Gr, 0) + 1;
-            const int n = (2 * Wd + 1) * n_full - (2 * Gd + 1) * n_guard;
-            const float noise = T * (1.0f / (float)max(n, 1));
-            const float cut = tile[(dl + Wd) * tw_ + x + Lp];
-            if ((r < Sp) && (n > 0) && (cut > p.alpha * noise)) {
-                atomicOr(&words[x], 1u << dl);
-                noise_map[((size_t)f * Cp + d0 + dl) * Sp + r] = noise;
-            }
+        const int n_full = min(r + Wr, Sp - 1) - max(r - Wr, 0) + 1;
+        const int n_guard = min(r + Gr, Sp - 1) - max(r - Gr, 0) + 1;
+        const int n = (2 * Wd + 1) * n_full - (2 * Gd + 1) * n_guard;
+        const float noise = T * (1.0f / (float)max(n, 1));
+        const float cut = tile[(dl + Wd) * tw_ + x + Lp];
+        if ((r < Sp) && (n > 0) && (cut > p.alpha * noise)) {
+            atomicOr(&words[x], 1u << dl);
+            noise_map[((size_t)f * Cp + d0 + dl) * Sp + r] = noise;
         }
     }
     __syncthreads();
@@ -198,7 +115,8 @@ __global__ void __launch_bounds__(kCfarNT) cfar_kernel(PlanDev p, const float *_
 // ---------------------------------------------------------------------------
 // K3, default geometry (guard 2x2, train 8x4), Sp % 64 == 0, Cp % 32 == 0: "walk" form.
 //
-// cfar_kernel above is instruction-bound (ncu: ~74 thread instructions per cell): independent 64 x 32 tiles re-stage
+// A tiled kernel like cfar_kernel above is instruction-bound (ncu, on its fully unrolled form for this window, which the
+// walk form replaced: ~74 thread instructions per cell): independent 64 x 32 tiles re-stage
 // 1.9x their cells as halo, and the column pass reads 22 scalar shared-memory words per 4 cells.  Here the window is
 // split the other way round.  With F13 / R8 = the 13-row Doppler sum of one range column and its 8-row ring (13 minus
 // the 5 guard rows),
@@ -1136,14 +1054,12 @@ static int cfar_smem_bytes(const PlanDev &p)
     return (th_ * tw_ + 2 * th_ * kCfarRS) * 4 + kCfarRT * 4;
 }
 
-// PlanDev.k3_variant (MMW_K3_VARIANT at mmw_create; profiles/sweep_variants.py, tests): 0 = pick by shape, 1 = always the tiled
-// kernel, 2/3/4 = walk kernel forced to 64- / 128- / 256-bin strips, +10 * nchunk to force the Doppler segment length
-
+// The default window takes the walk form (every plan_supported shape has Sp % 64 == 0 and Cp % 32 == 0); the tiled
+// cfar_kernel serves every other window.
 cudaError_t launch_cfar(const PlanDev &p, const float *pmap, uint32_t *mask, float *noise_map, int n_frames, int sm_count, cudaStream_t st)
 {
     const bool fixed = p.guard_r == 2 && p.guard_d == 2 && p.win_r_half == 10 && p.win_d_half == 6;
-    const int var = p.k3_variant;
-    if (fixed && p.Sp % 64 == 0 && p.Cp % 32 == 0 && var != 1) {
+    if (fixed && p.Sp % 64 == 0 && p.Cp % 32 == 0) {
         // walk form.  Longer Doppler segments amortise the 12-row run-in (28 input rows for the first 16 outputs, 16
         // after that), wider strips the 24-column halo; both are traded against having enough CTAs for every SM.
         const long long cells = (long long)n_frames * p.Sp * p.Cp;
@@ -1153,10 +1069,6 @@ cudaError_t launch_cfar(const PlanDev &p, const float *pmap, uint32_t *mask, flo
         if (p.Sp % 256 == 0 && cells / (256 * 32) >= want) rt = 256;
         int nchunk = 2;
         while (nchunk < 8 && p.Cp % (32 * nchunk) == 0 && cells / ((long long)rt * 32 * nchunk) >= want) nchunk *= 2;
-        if (var % 10 == 2) rt = 64;
-        if (var % 10 == 3 && p.Sp % 128 == 0) rt = 128;
-        if (var % 10 == 4 && p.Sp % 256 == 0) rt = 256;
-        if (var >= 10 && var / 10 % 2 == 0 && p.Cp % (16 * (var / 10)) == 0) nchunk = var / 10;
         switch (rt) {
         case 256: return run_cfar_walk<256, 3>(p, pmap, mask, noise_map, nchunk, n_frames, st);
         case 128: return run_cfar_walk<128, 5>(p, pmap, mask, noise_map, nchunk, n_frames, st);
@@ -1164,19 +1076,15 @@ cudaError_t launch_cfar(const PlanDev &p, const float *pmap, uint32_t *mask, flo
         }
     }
     const int bytes = cfar_smem_bytes(p);
-    static int configured_dev[kMaxDevices][2] = {{0}};
-    int *configured = configured_dev[current_device()];
-    if (bytes > configured[fixed]) {
-        cudaError_t e = fixed ? cudaFuncSetAttribute(cfar_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes)
-                              : cudaFuncSetAttribute(cfar_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    static int configured_dev[kMaxDevices] = {0};
+    int &configured = configured_dev[current_device()];
+    if (bytes > configured) {
+        cudaError_t e = cudaFuncSetAttribute(cfar_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
         if (e != cudaSuccess) return e;
-        configured[fixed] = bytes;
+        configured = bytes;
     }
     dim3 grid((p.Sp + kCfarRT - 1) / kCfarRT, p.Cp / kCfarDT, n_frames);
-    if (fixed)
-        cfar_kernel<true><<<grid, kCfarNT, bytes, st>>>(p, pmap, mask, noise_map);
-    else
-        cfar_kernel<false><<<grid, kCfarNT, bytes, st>>>(p, pmap, mask, noise_map);
+    cfar_kernel<<<grid, kCfarNT, bytes, st>>>(p, pmap, mask, noise_map);
     return cudaGetLastError();
 }
 
@@ -1206,8 +1114,9 @@ cudaError_t launch_detect(const PlanDev &p, const DetectBuffers &b, int n_frames
     if (e != cudaSuccess) return e;
     const bool wide = p.A >= kMeasWideA;
     // wide arrays, fused mode: one more Doppler FFT of the rows that have hits, then the angle spectra as FFTs
-    // (PlanDev.k4_variant = 1 keeps the per-detection kernel below: tests and profiles compare the two)
-    if ((wide || p.k4_variant == 2) && !p.keep_cube && b.rows != nullptr && b.snap != nullptr && p.k4_variant != 1) {
+    // (PlanDev.detect_path, mmw_set_detect_path, forces either path)
+    if ((wide || p.detect_path == MMW_DETECT_REFFT) && !p.keep_cube && b.rows != nullptr && b.snap != nullptr &&
+        p.detect_path != MMW_DETECT_PER_CELL) {
         const int rgrid = (dense_cap + 255) / 256 < sm_count * 4 ? (dense_cap + 255) / 256 : sm_count * 4;
         rows_kernel<<<rgrid < 1 ? 1 : rgrid, 256, 0, st>>>(p, b.keys, b.offsets, b.rows, b.ticket + 2, n_frames, dense_cap);
         e = cudaGetLastError();

@@ -55,31 +55,32 @@ __device__ __forceinline__ void sched_retire(unsigned int *ctr)
 // ---------------------------------------------------------------------------
 // K1: range FFT
 // ---------------------------------------------------------------------------
-template <int N, int BT, int NSTAGE, bool BASE = false>
+template <int N, int BT, bool BASE = false>
 struct RangeSmem {
     static constexpr int kStageStride = 4 * N + 16;                 // bytes per staged int16 row
     static constexpr int kOffTw = 16;
     static constexpr int kOffWin = kOffTw + 8 * N;
     static constexpr int kOffStage = kOffWin + 4 * N;
     static constexpr int kStageBytes = BT * kStageStride;
-    static constexpr int kOffBase = kOffStage + NSTAGE * kStageBytes;   // BASE: the tile's rows of the base frame, staged alongside
-    static constexpr int kOffWork = kOffBase + (BASE ? NSTAGE * kStageBytes : 0);
+    static constexpr int kOffBase = kOffStage + kStageBytes;            // BASE: the tile's rows of the base frame, staged alongside
+    static constexpr int kOffWork = kOffBase + (BASE ? kStageBytes : 0);
     static constexpr int kBytes = kOffWork + BT * (N + 1) * 8;
 };
 
 // PAIR: a thread runs butterflies n2 and n2+1 together (one 8-byte load yields both samples of an IIQQ group).
 // PAD : n_samples < N (zero padding needs a bound check per load); CT: compile-time n_chirps, 0 = run time.
-// NSTAGE = 1: one staging buffer, refilled behind pass 2; NSTAGE = 2: double buffer, refilled a whole tile ahead.
+// One staging buffer, refilled behind pass 2 (a double buffer refilled a whole tile ahead measured slower:
+// profiles/experiments/r1_k1_variants_sweep.log).
 // BASE: static-clutter removal — p.base_adc (one frame in capture format) is subtracted sample by sample, in integers,
 // before the window (the reference's base-frame subtraction, acceleration.cu:152-166, for every antenna).  The tile's
 // rows of the base frame are staged by the same TMA copies as the capture rows (they come from L2: the base frame is a
 // few MB read by every CTA); reading them with per-lane global loads instead costs 4x sector over-fetch and +70 % time.
-template <int N, int R1, int R2, int BT, int NW, bool PAIR, bool PAD, int CT, int NSTAGE, bool BASE>
-__global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, NSTAGE, BASE>::kBytes <= 226 * 1024 && NW <= 8) ? 2 : 1) range_fft_kernel(PlanDev p, const int16_t *__restrict__ adc, float2 *__restrict__ rs,
+template <int N, int R1, int R2, int BT, int NW, bool PAIR, bool PAD, int CT, bool BASE>
+__global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, BASE>::kBytes <= 226 * 1024 && NW <= 8) ? 2 : 1) range_fft_kernel(PlanDev p, const int16_t *__restrict__ adc, float2 *__restrict__ rs,
                                                             int n_tiles)
 {
     static_assert(R1 * R2 == N, "plan");
-    using L = RangeSmem<N, BT, NSTAGE, BASE>;
+    using L = RangeSmem<N, BT, BASE>;
     constexpr int NT = NW * 32;
     constexpr int SUBS = 32 / BT;
     constexpr int NSLOT = NW * SUBS;
@@ -99,12 +100,12 @@ __global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, NSTAGE, BASE>::
     const int C = CT ? CT : p.C;
     const int nct = (C + BT - 1) / BT;
 
-    auto issue = [&](int tile, int it) {    // one warp: stage the BT int16 rows of `tile` (the it-th tile of this CTA)
+    auto issue = [&](int tile) {            // one warp: stage the BT int16 rows of `tile`
         const int ct = tile % nct, fa = tile / nct;
         const int a = fa % A, f = fa / A;
         const int c0 = ct * BT;
         const int nrows = min(BT, C - c0);
-        uint64_t *b = &bar[it % NSTAGE];
+        uint64_t *b = &bar[0];
         if (lane == 0) {
             fence_proxy_async();
             mbar_arrive_expect_tx(b, (uint32_t)(nrows * S * 4) * (BASE ? 2u : 1u));
@@ -112,10 +113,10 @@ __global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, NSTAGE, BASE>::
         __syncwarp();
         if (lane < nrows) {
             const int16_t *src = adc + (((size_t)f * C + c0 + lane) * A + a) * (size_t)(2 * S);
-            bulk_g2s(stage + (it % NSTAGE) * L::kStageBytes + lane * L::kStageStride, src, (uint32_t)(S * 4), b);
+            bulk_g2s(stage + lane * L::kStageStride, src, (uint32_t)(S * 4), b);
             if constexpr (BASE) {
                 const int16_t *bsrc = p.base_adc + ((size_t)(c0 + lane) * A + a) * (size_t)(2 * S);
-                bulk_g2s(bstage + (it % NSTAGE) * L::kStageBytes + lane * L::kStageStride, bsrc, (uint32_t)(S * 4), b);
+                bulk_g2s(bstage + lane * L::kStageStride, bsrc, (uint32_t)(S * 4), b);
             }
         }
     };
@@ -123,17 +124,17 @@ __global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, NSTAGE, BASE>::
     // Tiles are handed out by a counter (PlanDev.sched), not by a fixed stride: a CTA that starts late — its SM was still held by
     // a kernel of another stream (another batch in flight, the exchange's merge kernel) — simply takes fewer tiles instead of
     // finishing its fixed share late.  The first tile of a CTA is blockIdx.x; the next one is fetched while pass 1 runs.
-    const bool DYN = NSTAGE == 1 && (p.sched_dynamic & 1);
+    const bool DYN = (p.sched_dynamic & 1) != 0;
     __shared__ int s_next[2];
     unsigned int *ctr = p.sched;                                      // [0] next tile - gridDim.x, [1] CTAs done
     if (tid == 0) {
         mbar_init(&bar[0], 1);
-        mbar_init(&bar[1], 1);
+        mbar_init(&bar[1], 1);                                        // not waited on since the double buffer went; kept: same machine code
         fence_mbar_init();
     }
     __syncthreads();
     int tile = blockIdx.x;
-    if (warp == 0 && tile < n_tiles) issue(tile, 0);
+    if (warp == 0 && tile < n_tiles) issue(tile);
     for (int i = tid; i < N; i += NT) tw[i] = p.tw1_r[i];
     for (int i = tid; i < N; i += NT) win[i] = i < S ? p.win_r[i] : 0.f;
     __syncthreads();
@@ -149,10 +150,9 @@ __global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, NSTAGE, BASE>::
         const float wdop = row_ok ? p.win_d[c0 + row] : 0.f;
         unsigned int fetched = 0u;
         if (DYN && tid == 0) fetched = atomicAdd(&ctr[0], 1u);        // answer needed after pass 1 only
-        if (NSTAGE == 2 && warp == 0 && tile + (int)gridDim.x < n_tiles) issue(tile + gridDim.x, it + 1);
-        mbar_wait(&bar[it % NSTAGE], (uint32_t)((it / NSTAGE) & 1));
-        const unsigned char *srow = stage + (it % NSTAGE) * L::kStageBytes + row * L::kStageStride;
-        const unsigned char *brow = BASE ? bstage + (it % NSTAGE) * L::kStageBytes + row * L::kStageStride : nullptr;
+        mbar_wait(&bar[0], (uint32_t)(it & 1));
+        const unsigned char *srow = stage + row * L::kStageStride;
+        const unsigned char *brow = BASE ? bstage + row * L::kStageStride : nullptr;
 
         // ---- pass 1: R2 butterflies of radix R1 over stride R2, reading the staged int16 rows ----
         if constexpr (PAIR) {
@@ -232,11 +232,11 @@ __global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, NSTAGE, BASE>::
         if (DYN && tid == 0) s_next[(it + 1) & 1] = (int)min(fetched + gridDim.x, (unsigned int)n_tiles);
         __syncthreads();
         const int next_tile = DYN ? s_next[(it + 1) & 1] : tile + (int)gridDim.x;
-        // single staging buffer: it is consumed now, prefetch the next tile behind pass 2.  (Refilling it earlier — as
+        // the staging buffer is consumed now: prefetch the next tile behind pass 2.  (Refilling it earlier — as
         // soon as the last warp has pulled its pass-1 inputs into registers — removes the wait on the copy but not a
         // microsecond of run time: the stall moves to the barrier, profiles/experiments/r1_k1_early_release.md.  L2 prefetch
         // hints for the tiles after that made it slower, r1_k1_l2_prefetch.log.)
-        if (NSTAGE == 1 && warp == 0 && next_tile < n_tiles) issue(next_tile, it + 1);
+        if (warp == 0 && next_tile < n_tiles) issue(next_tile);
 
         // ---- pass 2: R1 butterflies of radix R2 on contiguous runs; outputs go straight to HBM ----
         float2 *out = rs + (size_t)fa * (size_t)N * C + c0 + row;
@@ -891,10 +891,6 @@ __global__ void __launch_bounds__(256) power_sum_kernel(const float *__restrict_
     }
 }
 
-}  // namespace mmw
-#include "mmw_front.cuh"
-namespace mmw {
-
 // ---------------------------------------------------------------------------
 // export kernels (not on the hot path)
 // ---------------------------------------------------------------------------
@@ -970,30 +966,18 @@ static cudaError_t resident_ctas(K kernel, int threads, int smem_bytes, int *cta
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, kernel, threads, smem_bytes);
 }
 
-// PlanDev.ctas_per_sm_cap (MMW_CTAS_PER_SM at mmw_create; experiment): cap of resident CTAs per SM for the persistent FFT
-// kernels, so that the FFT kernels of two batches in flight can share every SM instead of taking turns
-// (profiles/experiments/r1_fft_corun.log)
-static int capped_per_sm(const PlanDev &p, int per_sm)
+// Grid of a persistent FFT kernel: every resident CTA slot, or fewer when there is less work than that
+static int persistent_grid(int per_sm, long long work_items)
 {
-    return p.ctas_per_sm_cap > 0 && p.ctas_per_sm_cap < per_sm ? p.ctas_per_sm_cap : per_sm;
-}
-
-// Grid of a persistent FFT kernel: every resident CTA slot, less PlanDev.reserve_ctas (mmw_reserve_ctas).  The FFT kernels
-// fill an SM's register file, so a kernel of another stream that arrives while one runs — the NCCL kernel of the sharded
-// exchange, the merge kernel, the detection kernels of another batch in flight — finds no SM to start on until an FFT CTA
-// retires; slots left free let it start at once, at the price of reserve / (2 x 148) of the FFT throughput.
-static int persistent_grid(const PlanDev &p, int per_sm, long long work_items)
-{
-    long long slots = (long long)capped_per_sm(p, per_sm) * sm_count();
-    if (p.reserve_ctas > 0) slots = slots - p.reserve_ctas > sm_count() ? slots - p.reserve_ctas : (slots > sm_count() ? sm_count() : slots);
+    const long long slots = (long long)per_sm * sm_count();
     return (int)(work_items < slots ? work_items : slots);
 }
 
-template <int N, int R1, int R2, int BT, int NW, bool PAIR, bool PAD, int CT, int NSTAGE, bool BASE = false>
+template <int N, int R1, int R2, int BT, int NW, bool PAIR, bool PAD, int CT, bool BASE = false>
 static cudaError_t run_range_t(const PlanDev &p, const int16_t *adc, float2 *rs, int n_frames, cudaStream_t st)
 {
-    auto k = range_fft_kernel<N, R1, R2, BT, NW, PAIR, PAD, CT, NSTAGE, BASE>;
-    constexpr int bytes = RangeSmem<N, BT, NSTAGE, BASE>::kBytes;
+    auto k = range_fft_kernel<N, R1, R2, BT, NW, PAIR, PAD, CT, BASE>;
+    constexpr int bytes = RangeSmem<N, BT, BASE>::kBytes;
     static int per_sm_dev[kMaxDevices] = {0};
     int &per_sm = per_sm_dev[current_device()];
     if (!per_sm) {
@@ -1003,26 +987,26 @@ static cudaError_t run_range_t(const PlanDev &p, const int16_t *adc, float2 *rs,
     }
     const int nct = (p.C + BT - 1) / BT;
     const long long tiles = (long long)n_frames * p.A * nct;
-    const int grid = persistent_grid(p, per_sm, tiles);
+    const int grid = persistent_grid(per_sm, tiles);
     k<<<grid, NW * 32, bytes, st>>>(p, adc, rs, (int)tiles);
     return cudaGetLastError();
 }
 
 // picks the PAD / compile-time-chirps specialisation
 // BBT / BNW: tile rows and warps of the static-clutter-removal instantiation (the second staging buffer has to fit)
-template <int N, int R1, int R2, int BT, int NW, bool PAIR, int CT0, int CT1, int NSTAGE = 1, int BBT = BT, int BNW = NW>
+template <int N, int R1, int R2, int BT, int NW, bool PAIR, int CT0, int CT1, int BBT = BT, int BNW = NW>
 static cudaError_t run_range(const PlanDev &p, const int16_t *adc, float2 *rs, int n_frames, cudaStream_t st)
 {
     if (p.base_adc != nullptr) {          // static-clutter removal: one generic instantiation per padding mode
-        if (p.S == N) return run_range_t<N, R1, R2, BBT, BNW, PAIR, false, 0, NSTAGE, true>(p, adc, rs, n_frames, st);
-        return run_range_t<N, R1, R2, BBT, BNW, PAIR, true, 0, NSTAGE, true>(p, adc, rs, n_frames, st);
+        if (p.S == N) return run_range_t<N, R1, R2, BBT, BNW, PAIR, false, 0, true>(p, adc, rs, n_frames, st);
+        return run_range_t<N, R1, R2, BBT, BNW, PAIR, true, 0, true>(p, adc, rs, n_frames, st);
     }
     if (p.S == N) {
-        if (CT0 && p.C == CT0) return run_range_t<N, R1, R2, BT, NW, PAIR, false, CT0, NSTAGE>(p, adc, rs, n_frames, st);
-        if (CT1 && p.C == CT1) return run_range_t<N, R1, R2, BT, NW, PAIR, false, CT1, NSTAGE>(p, adc, rs, n_frames, st);
-        return run_range_t<N, R1, R2, BT, NW, PAIR, false, 0, NSTAGE>(p, adc, rs, n_frames, st);
+        if (CT0 && p.C == CT0) return run_range_t<N, R1, R2, BT, NW, PAIR, false, CT0>(p, adc, rs, n_frames, st);
+        if (CT1 && p.C == CT1) return run_range_t<N, R1, R2, BT, NW, PAIR, false, CT1>(p, adc, rs, n_frames, st);
+        return run_range_t<N, R1, R2, BT, NW, PAIR, false, 0>(p, adc, rs, n_frames, st);
     }
-    return run_range_t<N, R1, R2, BT, NW, PAIR, true, 0, NSTAGE>(p, adc, rs, n_frames, st);
+    return run_range_t<N, R1, R2, BT, NW, PAIR, true, 0>(p, adc, rs, n_frames, st);
 }
 
 template <int N, int R1, int R2, int BT, int NW, bool PAD, int SPT, int NSTAGE, bool INPLACE>
@@ -1038,7 +1022,7 @@ static cudaError_t run_doppler_t(const PlanDev &p, const float2 *rs, float2 *cub
         if (per_sm < 1) return cudaErrorLaunchOutOfResources;
     }
     const long long tiles = (long long)n_frames * (p.Sp / BT);
-    const int grid = persistent_grid(p, per_sm, tiles);
+    const int grid = persistent_grid(per_sm, tiles);
     k<<<grid, NW * 32, bytes, st>>>(p, rs, cube, pmap, (int)tiles);
     return cudaGetLastError();
 }
@@ -1058,7 +1042,7 @@ static cudaError_t run_doppler_warp_t(const PlanDev &p, const float2 *rs, float 
     }
     const long long tiles = (long long)n_frames * (p.Sp / L::kRows);
     const long long want = (tiles + NW - 1) / NW;
-    const int grid = persistent_grid(p, per_sm, want);
+    const int grid = persistent_grid(per_sm, want);
     k<<<grid, NW * 32, bytes, st>>>(p, rs, pmap, (int)tiles);
     return cudaGetLastError();
 }
@@ -1084,81 +1068,6 @@ static cudaError_t run_doppler(const PlanDev &p, const float2 *rs, float2 *cube,
     return run_doppler_t<N, R1, R2, BT, NW, true, 0, NSTAGE, INPLACE>(p, rs, cube, pmap, n_frames, st);
 }
 
-// ---------------------------------------------------------------------------
-// fused front: K1 and K2 as the two roles of one cooperative persistent kernel (mmw_front.cuh)
-// ---------------------------------------------------------------------------
-template <int SN, int SR1, int SR2, int BT, int DN, int DR1, int DR2, int NW>
-static cudaError_t run_front_fused(const PlanDev &p, const int16_t *adc, float2 *rs, float *pmap, int n_frames, unsigned int *sync,
-                                   cudaStream_t st)
-{
-    const bool pads = p.S != SN, padc = p.C != DN;
-    using KernelT = void (*)(PlanDev, FrontArgs);
-    KernelT k = pads ? (padc ? front_fused_kernel<SN, SR1, SR2, BT, true, DN, DR1, DR2, true, NW>
-                             : front_fused_kernel<SN, SR1, SR2, BT, true, DN, DR1, DR2, false, NW>)
-                     : (padc ? front_fused_kernel<SN, SR1, SR2, BT, false, DN, DR1, DR2, true, NW>
-                             : front_fused_kernel<SN, SR1, SR2, BT, false, DN, DR1, DR2, false, NW>);
-    constexpr int bytes = FrontSmem<SN, BT, DN, DR1, DR2, NW>::kBytes;
-    static int per_sm_dev[kMaxDevices][4] = {{0}};
-    int &per_sm = per_sm_dev[current_device()][(pads ? 2 : 0) + (padc ? 1 : 0)];
-    if (!per_sm) {
-        cudaError_t e = resident_ctas(k, NW * 32, bytes, &per_sm);
-        if (e != cudaSuccess) return e;
-        if (per_sm < 2) { per_sm = 0; return cudaErrorLaunchOutOfResources; }
-        if (per_sm > 512 / (NW * 32)) per_sm = 512 / (NW * 32);     // 16 warps per SM: what 128 registers per thread allow
-    }
-    const int sms = sm_count();
-    const int nrt = p.Sp / DopplerWarp<DN, DR1, DR2>::kRows;          // consumer tiles (= warps) per frame
-    const int nct = (p.C + BT - 1) / BT;                              // producer tiles per slab
-    int FG = (sms * 8) / nrt;                                         // frames the consumer role holds at a time: 8 of an SM's 16 warps
-    if (FG < 1) return cudaErrorInvalidConfiguration;
-    if (FG > n_frames) FG = n_frames;
-    FrontArgs g;
-    g.adc = adc; g.rs = rs; g.pmap = pmap;
-    g.produced = sync; g.consumed = sync + (size_t)n_frames * p.A;
-    g.n_frames = n_frames; g.FG = FG; g.stats = p.front_stats;
-    g.n_consumer_ctas = (FG * nrt + NW - 1) / NW;
-    const long long tiles = (long long)n_frames * p.A * nct;
-    long long nprod = (long long)per_sm * sms - g.n_consumer_ctas;
-    if (nprod > tiles) nprod = tiles;
-    if (nprod < 1) return cudaErrorInvalidConfiguration;
-    // slabs the producers hold in flight (a tile in work + one staged per CTA) + two antenna steps of the consumer group
-    const int inflight = (int)((2 * nprod + nct - 1) / nct);
-    g.window = p.front_window > 0 ? p.front_window : inflight + 2 * FG;
-    if (g.window < FG + 1) g.window = FG + 1;
-    cudaError_t e = cudaMemsetAsync(sync, 0, (size_t)2 * n_frames * p.A * sizeof(unsigned int), st);
-    if (e != cudaSuccess) return e;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(g.n_consumer_ctas + nprod));
-    cfg.blockDim = dim3(NW * 32);
-    cfg.dynamicSmemBytes = bytes;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeCooperative;                      // every CTA resident at once: the roles wait for each other
-    attr[0].val.cooperative = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, k, p, g);
-}
-
-bool front_fused_supported(const PlanDev &p, int n_frames)
-{
-    if (p.keep_cube || p.base_adc != nullptr || p.A < 1) return false;
-    if (!((p.Sp == 512 && p.Cp == 256) || (p.Sp == 256 && p.Cp == 128))) return false;
-    // enough producer tiles to fill the grid a few times over; small batches keep the antenna-split path
-    return (long long)n_frames * p.A * ((p.C + 15) / 16) >= 8LL * sm_count();
-}
-
-cudaError_t launch_front_fused(const PlanDev &p, const int16_t *adc, float2 *rs, float *pmap, int n_frames, unsigned int *sync, cudaStream_t st)
-{
-    if (p.Sp == 512 && p.Cp == 256) {
-        // MMW_FRONT=3: 8-chirp producer tiles, 4 warps per CTA, four CTAs per SM (smaller barrier domains)
-        if (p.front_variant == 3) return run_front_fused<512, 16, 32, 8, 256, 16, 16, 4>(p, adc, rs, pmap, n_frames, sync, st);
-        return run_front_fused<512, 16, 32, 16, 256, 16, 16, 8>(p, adc, rs, pmap, n_frames, sync, st);
-    }
-    if (p.Sp == 256 && p.Cp == 128) return run_front_fused<256, 16, 16, 16, 128, 8, 16, 8>(p, adc, rs, pmap, n_frames, sync, st);
-    return cudaErrorInvalidValue;
-}
-
 bool plan_supported(int Sp, int Cp, const char **why)
 {
     auto ok = [](int n) { return n == 64 || n == 128 || n == 256 || n == 512 || n == 1024; };
@@ -1175,26 +1084,20 @@ cudaError_t launch_range_fft(const PlanDev &p, const int16_t *adc, float2 *rs, i
     switch (p.Sp) {
     case 64:   return run_range<64, 8, 8, 16, 4, true, 0, 0>(p, adc, rs, n_frames, st);
     case 128:  return run_range<128, 8, 16, 16, 4, true, 128, 0>(p, adc, rs, n_frames, st);
-    // double-buffered staging (NSTAGE = 2) and BT = 8 tiles were measured slower for 256 and 512 points
+    // double-buffered staging and BT = 8 tiles were measured slower for 256 and 512 points
     // (profiles/experiments/r1_k1_variants_sweep.log)
     // Tile height = bytes per range row in one corner-turned store: a 1 : 2 read:write mover reaches 5.2 TB/s with 128-byte pieces
     // and 5.6-5.7 TB/s with 256-byte ones (profiles/membench_r1.txt).  256 points: 32-row tiles still fit two CTAs of 8 warps per SM
     // and measured 4.5 % faster than 16-row tiles with three CTAs of 4 warps (cfg2 0.293 -> 0.280 ms).  512 points: a 32-row tile
     // needs 203 KB, one CTA of 16 warps per SM, and loses more to the barrier between the passes than the stores gain (0.224 ->
-    // 0.238 ms).  MMW_K1_VARIANT = 5 / 6 force 32- / 16-row tiles (profiles/experiments/r1_k1_tile_height.log).  Re-measured with tiles
-    // from the counter (profiles/r2/sweep_k1_tiles_dynamic.log): same ranking, 8-row tiles at 512 points (four CTAs of 4 warps) 0.225 vs 0.201 ms.
-    case 256:
-        if (p.k1_variant == 6) return run_range<256, 16, 16, 16, 4, true, 128, 0>(p, adc, rs, n_frames, st);
-        return run_range<256, 16, 16, 32, 8, true, 128, 0, 1, 16, 4>(p, adc, rs, n_frames, st);
-    case 512:
-        if (p.k1_variant == 5) return run_range<512, 16, 32, 32, 16, true, 256, 0, 1, 8, 4>(p, adc, rs, n_frames, st);
-        return run_range<512, 16, 32, 16, 8, true, 256, 0, 1, 8, 4>(p, adc, rs, n_frames, st);
+    // 0.238 ms), profiles/experiments/r1_k1_tile_height.log.  Re-measured with tiles from the counter
+    // (profiles/r2/sweep_k1_tiles_dynamic.log): same ranking, 8-row tiles at 512 points (four CTAs of 4 warps) 0.225 vs 0.201 ms.
+    case 256:  return run_range<256, 16, 16, 32, 8, true, 128, 0, 16, 4>(p, adc, rs, n_frames, st);
+    case 512:  return run_range<512, 16, 32, 16, 8, true, 256, 0, 8, 4>(p, adc, rs, n_frames, st);
     // 1024 points: a 16-row tile needs 209 KB (one CTA per SM).  With 8 warps it lost 2.4 % to 8-row tiles at two CTAs per SM
     // (profiles/experiments/r1_cfg4_tile_sweep.log); with 16 warps it wins 1-4 % (64-byte store pieces are the worst case of
-    // profiles/membench_r1.txt: 4.2 TB/s), profiles/experiments/r1_k1_tile_height.log.  MMW_K1_VARIANT = 6: the 8-row shape.
-    case 1024:
-        if (p.k1_variant == 6) return run_range<1024, 32, 32, 8, 8, false, 512, 0, 1, 4, 4>(p, adc, rs, n_frames, st);
-        return run_range<1024, 32, 32, 16, 16, false, 512, 0, 1, 4, 4>(p, adc, rs, n_frames, st);
+    // profiles/membench_r1.txt: 4.2 TB/s), profiles/experiments/r1_k1_tile_height.log.
+    case 1024: return run_range<1024, 32, 32, 16, 16, false, 512, 0, 4, 4>(p, adc, rs, n_frames, st);
     default:   return cudaErrorInvalidValue;
     }
 }
@@ -1205,29 +1108,14 @@ cudaError_t launch_doppler_fft(const PlanDev &p, const float2 *rs, float2 *cube,
 {
     switch (p.Cp) {
     case 64:   return run_doppler<64, 8, 8, 16, 4, 0, 0>(p, rs, cube, pmap, n_frames, st);
-    case 128: {
-        const int v = p.k2_variant;
-        // tile-shape experiments kept selectable for profiles/sweep_variants.py (results: profiles/experiments/)
-        // warp-private tiles (K2w) are slower at 128 points (4 rows x 8 lanes, two butterflies per thread): 0.222 vs 0.207 ms
-        if (v == 11 && !cube) return run_doppler_warp<128, 8, 16, 8, 256, 2>(p, rs, pmap, n_frames, st);
-        if (v == 1) return run_doppler<128, 8, 16, 8, 4, 256, 128, 2>(p, rs, cube, pmap, n_frames, st);
-        if (v == 6) return run_doppler<128, 8, 16, 16, 4, 256, 128, 3, true>(p, rs, cube, pmap, n_frames, st);
-        return run_doppler<128, 8, 16, 16, 4, 256, 128>(p, rs, cube, pmap, n_frames, st);
-    }
-    case 256: {
-        const int v = p.k2_variant;
-        if (v == 1) return run_doppler<256, 16, 16, 8, 4, 512, 0, 2>(p, rs, cube, pmap, n_frames, st);
-        if (v == 6) return run_doppler<256, 16, 16, 16, 8, 512, 0, 3, true>(p, rs, cube, pmap, n_frames, st);
-        if (v == 10 && !cube) return run_doppler_warp<256, 16, 16, 8, 512, 3>(p, rs, pmap, n_frames, st);
-        if (v == 13 && !cube) return run_doppler_warp<256, 16, 16, 10, 512, 2>(p, rs, pmap, n_frames, st);
-        if (v == 14 && !cube) return run_doppler_warp<256, 16, 16, 12, 512, 2>(p, rs, pmap, n_frames, st);
-        if (v == 15 && !cube) return run_doppler_warp<256, 16, 16, 6, 512, 2, 3>(p, rs, pmap, n_frames, st);
-        if (v == 16 && !cube) return run_doppler_warp<256, 16, 16, 5, 512, 2, 4>(p, rs, pmap, n_frames, st);
-        if (v == 17 && !cube) return run_doppler_warp<256, 16, 16, 6, 512, 3, 3>(p, rs, pmap, n_frames, st);
+    // Other tile shapes, in-place staging and other warp counts were swept and lost: profiles/experiments/r1_k2_variants_sweep.log,
+    // profiles/r2/sweep_k2_occupancy.log, profiles/r2/sweep_k2_warp_512_128.log.
+    // 128 points: warp-private tiles (K2w, 4 rows x 8 lanes, two butterflies per thread) are slower: 0.222 vs 0.207 ms
+    case 128:  return run_doppler<128, 8, 16, 16, 4, 256, 128>(p, rs, cube, pmap, n_frames, st);
+    case 256:
         // fused mode (power map only): warp-private tiles, 0.156 vs 0.171 ms on cfg3 (profiles/experiments/r1_k2_warp_private.log)
-        if (v != 12 && !cube) return run_doppler_warp<256, 16, 16, 8, 512, 2>(p, rs, pmap, n_frames, st);
+        if (!cube) return run_doppler_warp<256, 16, 16, 8, 512, 2>(p, rs, pmap, n_frames, st);
         return run_doppler<256, 16, 16, 16, 8, 512, 0>(p, rs, cube, pmap, n_frames, st);
-    }
     // 512 points: 8-row tiles, in place, three staging buffers = 103 KB, two CTAs per SM: 0.76 ms against 1.00 ms for the
     // 16-row double-buffered shape (201 KB, one CTA per SM) on the cfg4 cube (profiles/experiments/r1_cfg4_tile_sweep.log)
     // (warp-private tiles at 512 points — 2 rows x 16 lanes, two radix-16 butterflies per lane in pass 1, one radix-32 in pass 2,

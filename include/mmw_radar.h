@@ -295,12 +295,6 @@ int mmw_exchange_put(mmw_exchange *x);                                    /* on 
 int mmw_exchange_merge(mmw_exchange *x, const void **merged_block);       /* rank 0: [32-byte header | ordered records], device */
 int mmw_exchange_wait(mmw_exchange *x, void *cuda_stream, const void **merged_block);   /* rank 0: stream waits for the last merge */
 
-/* Diagnostics of the fused front kernel (stages 1 and 2 as two roles of one kernel): with MMW_FRONT_STATS=1 in the
- * environment at mmw_create, every CTA of the last launch leaves 8 uint64: {SM id | role << 32 (1 = range, 0 = Doppler),
- * start ns, end ns, ns spent waiting for the other role, tiles / steps done, 0, 0, 0}.  Copies up to max_ctas records;
- * returns the number copied, MMW_ERR_STATE without the switch. */
-int mmw_front_stats(mmw_ctx *ctx, unsigned long long *out, int max_ctas);
-
 #ifdef __cplusplus
 }
 #endif

@@ -13,14 +13,12 @@ import __graft_entry__ as entry  # noqa: E402
 pkg = entry.load_package()
 S, C, A = 512, 256, 12
 dev = torch.device("cuda", 0)
-for v2 in (0, 1):
-    os.environ["MMW_K2_VARIANT"] = str(v2)
-    for F in (2, 4, 6, 8, 16, 64):
-        adc = pkg.synth.cube_batch_torch(F, S, C, A, dev, cfg=3)
-        with pkg.RadarContext(S, C, A, F) as ctx:
-            ctx.time_device(adc, F, 3)
-            tot, st = ctx.time_device(adc, F, 50, per_stage=True)
-            n = 50
-            print(f"k2v={v2} F={F:3d} rs={F * 12.58:.0f} MB: range {st[0] / n / F * 1e3:.2f} us/frame, doppler {st[1] / n / F * 1e3:.2f} us/frame, "
-                  f"cfar {st[2] / n * 1e3:.1f} us, detect {st[3] / n * 1e3:.1f} us, batch {tot / n * 1e3:.1f} us", flush=True)
-        del adc
+for F in (2, 4, 6, 8, 16, 64):
+    adc = pkg.synth.cube_batch_torch(F, S, C, A, dev, cfg=3)
+    with pkg.RadarContext(S, C, A, F) as ctx:
+        ctx.time_device(adc, F, 3)
+        tot, st = ctx.time_device(adc, F, 50, per_stage=True)
+        n = 50
+        print(f"F={F:3d} rs={F * 12.58:.0f} MB: range {st[0] / n / F * 1e3:.2f} us/frame, doppler {st[1] / n / F * 1e3:.2f} us/frame, "
+              f"cfar {st[2] / n * 1e3:.1f} us, detect {st[3] / n * 1e3:.1f} us, batch {tot / n * 1e3:.1f} us", flush=True)
+    del adc

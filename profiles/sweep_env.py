@@ -1,6 +1,6 @@
 """Stage times of a bench workload under different values of one environment switch read at mmw_create
-(MMW_K1_VARIANT, MMW_K2_VARIANT, MMW_K3_VARIANT, MMW_K4_VARIANT, MMW_FRONT, ...).
-    python profiles/sweep_env.py cfg3 MMW_K2_VARIANT=0,13,14"""
+(MMW_SCHED: how the persistent FFT kernels take their tiles).
+    python profiles/sweep_env.py cfg3 MMW_SCHED=0,1,3"""
 import os
 import sys
 

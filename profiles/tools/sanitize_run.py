@@ -1,5 +1,5 @@
-"""Small self-checking run sized for compute-sanitizer (memcheck / racecheck / synccheck): the chain on a small cube with every
-CFAR kernel form, submit/wait, graph mode with advancing frame offsets, the wide-array path (selective Doppler re-FFT + angle
+"""Small self-checking run sized for compute-sanitizer (memcheck / racecheck / synccheck): the chain on a small cube with both
+CFAR kernels (the walk form of the default window, the tiled one of another window), submit/wait, graph mode with advancing frame offsets, the wide-array path (selective Doppler re-FFT + angle
 FFT) and the warp-private Doppler kernel, and one legacy frame through both legacy kernels (the 8-CTA DSMEM cluster included).
     [compute-sanitizer --tool memcheck|racecheck|synccheck] python profiles/tools/sanitize_run.py"""
 import os
@@ -14,19 +14,13 @@ import __graft_entry__ as entry  # noqa: E402
 pkg = entry.load_package()
 S, C, A, F = 256, 128, 4, 2
 adc = pkg.synth.cube_batch(F, S, C, A, cfg=3, n_targets=5)
-ref = None
-for var in (1, 22, 43, 84, 0):
-    os.environ["MMW_K3_VARIANT"] = str(var)
-    with pkg.RadarContext(S, C, A, F) as ctx:
+for window in ({}, {"cfar_guard": (1, 3), "cfar_train": (5, 2)}):
+    with pkg.RadarContext(S, C, A, F, **window) as ctx:
         dets, _ = ctx.process_host(adc, F)
         ctx.submit_host(adc, F)
         again, _ = ctx.wait()
     assert again.tobytes() == dets.tobytes()
-    cells = [(int(d["frame"]), int(d["range_bin"]), int(d["doppler_bin"])) for d in dets]
-    ref = ref or cells
-    assert cells == ref, var
-    print("k3 variant", var, len(dets), "detections")
-os.environ.pop("MMW_K3_VARIANT")
+    print("CFAR window", window or "default", len(dets), "detections")
 with pkg.RadarContext(512, 64, 12, 1) as ctx:                       # 128-bin strips of a 512-bin map, one frame
     print("512 x 64 x 12:", len(ctx.process_host(pkg.synth.cube_batch(1, 512, 64, 12, cfg=3, n_targets=5), 1)[0]), "detections")
 with pkg.RadarContext(256, 256, 2, 4) as ctx:                       # 256-point Doppler FFT, fused: the warp-private kernel (in-place pass 1)

@@ -1,7 +1,7 @@
 """A memcheck of our own: contexts created with MMW_GUARD=1 bracket every device buffer they own with 4 KB guard bands
 (include/mmw_radar.h: mmw_check_guards), and after driving every kernel form of the chain — ragged and padded shapes, fused
 mode and cube mode, the antenna-split path of small batches, graph mode, static-clutter removal, the wide-array paths
-(selective Doppler re-FFT, measure_wide_kernel), the fused front, detection-capacity overflow, full batches that end exactly
+(selective Doppler re-FFT, measure_wide_kernel), detection-capacity overflow, full batches that end exactly
 at the buffers' last byte — not one guard byte may have changed.  compute-sanitizer is closed on this pool
 (profiles/r2/compute_sanitizer_refused.log); this catches out-of-bounds WRITES of any kernel, to the byte.  The reference's
 own kernels would not pass (acceleration.cu:117-150 reads out of bounds, :152-166 leaves element 12 800 unwritten)."""
@@ -67,24 +67,6 @@ def test_no_kernel_writes_outside_its_buffers(pkg, guard_env, S, C, A, F, keep, 
             ctx.doppler_cube(0)
         bad = ctx.check_guards()
     assert bad == 0, pkg.api.last_error()
-
-
-@pytest.mark.parametrize("front", ["2"])
-def test_fused_front_stays_inside_its_buffers(pkg, guard_env, front):
-    old = os.environ.get("MMW_FRONT")
-    os.environ["MMW_FRONT"] = front
-    try:
-        S, C, A, F = 512, 256, 12, 8
-        adc = pkg.synth.cube_batch(F, S, C, A, cfg=3, n_targets=6)
-        with pkg.RadarContext(S, C, A, F) as ctx:
-            ctx.process_host(adc, F)
-            ctx.process_host(adc[:3], 3)
-            assert ctx.check_guards() == 0, pkg.api.last_error()
-    finally:
-        if old is None:
-            os.environ.pop("MMW_FRONT", None)
-        else:
-            os.environ["MMW_FRONT"] = old
 
 
 def test_guard_check_sees_a_stray_write(pkg, guard_env):

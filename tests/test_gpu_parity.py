@@ -142,38 +142,65 @@ def test_cfar_geometries(pkg, orc, guard, train, alpha):
             assert abs(d["noise"] - by[k]["noise"]) <= NOISE_RTOL * by[k]["noise"]
 
 
+def _walk_form(F, Sp, Cp, sm_count):
+    """launch_cfar's rule for the default window: (range bins per strip, Doppler segments of 16 bins per CTA)"""
+    cells, want = F * Sp * Cp, 8 * sm_count
+    rt = 64
+    if Sp % 128 == 0 and cells // (128 * 32) >= want:
+        rt = 128
+    if Sp % 256 == 0 and cells // (256 * 32) >= want:
+        rt = 256
+    nchunk = 2
+    while nchunk < 8 and Cp % (32 * nchunk) == 0 and cells // (rt * 32 * nchunk) >= want:
+        nchunk *= 2
+    return rt, nchunk
+
+
+@pytest.fixture(scope="module")
+def sm_count(pkg):
+    with pkg.RadarContext(64, 64, 1, 1) as ctx:
+        return ctx.info.sm_count
+
+
 @pytest.mark.parametrize("variant", [1, 22, 42, 82, 23, 43, 83, 24, 44, 84])
-def test_cfar_kernel_forms_agree_with_oracle(pkg, orc, cases, variant, monkeypatch):
-    """Every compiled form of K3 for the default geometry — the tiled kernel (1) and the walk kernel with 64- / 128- /
-    256-bin strips (2 / 3 / 4) and Doppler segments of 32 / 64 / 128 bins (+ 10 * nchunk) — against the oracle: same mask
-    away from threshold cells, and the noise estimate of every detection (the fp32 power map itself differs from the
-    fp64 one by more than the kernels differ from each other: profiles/sweep_k3.py compares the forms directly, 4e-7)."""
-    shape = (256, 128, 4)
-    S, C, A = shape
-    F, adc, wr, wd, ref = cases[shape]
-    near = _near_threshold(ref, 15.0)
-    monkeypatch.setenv("MMW_K3_VARIANT", str(variant))
-    with pkg.RadarContext(S, C, A, F) as ctx:
+def test_cfar_kernel_forms_agree_with_oracle(pkg, orc, sm_count, variant):
+    """Every form of K3 against the oracle's CFAR on the GPU's own power map: same mask away from threshold cells (the
+    clamped range edges included) and the noise estimate of every detection.  The forms are numbered as in the sweep
+    records (profiles/experiments/r1_cfar_walk_sweep.log): k + 10 * nchunk is the walk kernel with 64- / 128- / 256-bin
+    strips (k = 2 / 3 / 4) and Doppler segments of nchunk x 16 bins, reached through the batch size F for which
+    launch_cfar's rule picks it on this GPU (a few synthetic frames tiled to F); 1 is the tiled kernel, which serves every
+    window but the default one."""
+    if variant == 1:
+        S, C, F, train = 256, 128, 2, (8, 5)
+    else:
+        form = ({2: 64, 3: 128, 4: 256}[variant % 10], variant // 10)
+        S, C, F = next((S, C, F) for (S, C) in ((256, 128), (64, 256), (128, 256)) for F in range(1, 64 * sm_count)
+                       if _walk_form(F, S, C, sm_count) == form)
+        train = (8, 4)
+    base = pkg.synth.cube_batch(3, S, C, 1, cfg=3, n_targets=6)
+    adc = np.ascontiguousarray(base[np.arange(F) % 3])
+    with pkg.RadarContext(S, C, 1, F, cfar_train=train) as ctx:
         dets, overflow = ctx.process_host(adc, F)
-        masks = [ctx.cfar_mask(f) for f in range(F)]
-    for f in range(F):
-        assert not ((masks[f] != ref["mask"][f]) & ~near[f]).any()
+        assert not overflow
+        frames = sorted({0, F // 2, F - 1})
+        got = {f: (ctx.power_map(f), ctx.cfar_mask(f)) for f in frames}
+    for f in frames:
+        P, mask = got[f]
+        ref_mask, ref_noise = orc.cfar(P, train=train)
+        thr = 15.0 * ref_noise
+        near = np.abs(P - thr) <= NEAR * thr
+        assert not ((mask != ref_mask) & ~near).any(), f"frame {f}: CFAR cells differ away from threshold"
         for edge in (np.r_[0:12], np.r_[S - 12:S]):                      # clamped range rows; all Doppler columns incl. the wrap
-            assert not ((masks[f][edge] != ref["mask"][f][edge]) & ~near[f][edge]).any()
-    by = {(int(d["frame"]), int(d["range_bin"]), int(d["doppler_bin"])): d for d in ref["dets"]}
-    assert len(dets) > 0 and not overflow
-    hit = 0
-    for d in dets:
-        k = (int(d["frame"]), int(d["range_bin"]), int(d["doppler_bin"]))
-        if k in by:
-            hit += 1
-            assert abs(d["noise"] - by[k]["noise"]) <= NOISE_RTOL * by[k]["noise"]
-    assert hit >= len(dets) - int(near.sum())
+            assert not ((mask[edge] != ref_mask[edge]) & ~near[edge]).any(), f"frame {f}: clamped range edge differs"
+        d = dets[dets["frame"] == f]
+        assert len(d) == int(mask.sum()) > 0
+        r, c = d["range_bin"].astype(np.int64), d["doppler_bin"].astype(np.int64)
+        assert np.all(np.abs(d["noise"] - ref_noise[r, c]) <= NOISE_RTOL * ref_noise[r, c]), f"frame {f}: noise estimate"
 
 
-def test_wide_array_paths_agree(pkg, orc, monkeypatch):
+def test_wide_array_paths_agree(pkg, orc):
     """A >= 32 in fused mode: the selective Doppler re-FFT + angle FFT path (default) against the per-detection kernel it
-    replaces (MMW_K4_VARIANT=1 at context creation: direct Doppler DFT + angle DFT per detection) and against cube mode:
+    replaces (mmw_set_detect_path(MMW_DETECT_PER_CELL): direct Doppler DFT + angle DFT per detection) and against cube mode:
     same cells, powers, noise and flags bit for bit; angle bins identical away from ties of the angle spectrum."""
     S, C, A, F = 128, 64, 96, 3
     adc = pkg.synth.cube_batch(F, S, C, A, cfg=13, n_targets=6)
@@ -182,11 +209,10 @@ def test_wide_array_paths_agree(pkg, orc, monkeypatch):
     with pkg.RadarContext(S, C, A, F) as ctx:
         new, ov = ctx.process_host(adc, F)
         assert not ov and ctx.info.kernels_per_batch == 7
-    monkeypatch.setenv("MMW_K4_VARIANT", "1")
     with pkg.RadarContext(S, C, A, F) as ctx:
+        ctx.set_detect_path(pkg.api.DETECT_PER_CELL)
         old, _ = ctx.process_host(adc, F)
         assert ctx.info.kernels_per_batch == 5
-    monkeypatch.delenv("MMW_K4_VARIANT")
     with pkg.RadarContext(S, C, A, F, keep_doppler_cube=True) as ctx:
         cube, _ = ctx.process_host(adc, F)
     key = lambda d: (d["frame"].astype(np.int64) << 32) | (d["range_bin"].astype(np.int64) << 16) | d["doppler_bin"]
@@ -410,54 +436,54 @@ def test_chain_matches_numpy_golden_fixture(pkg, golden_dir):
                 assert n_checked > 0
 
 
-@pytest.mark.parametrize("shape,variants", [((512, 256, 12), [1, 6, 10, 12, 13, 14, 15, 16, 17]), ((256, 128, 4), [1, 6, 11]),
-                                            ((500, 130, 2), [10, 13, 17])])
-def test_doppler_kernel_forms_give_the_same_bits(pkg, shape, variants, monkeypatch):
-    """Every selectable form of K2 (MMW_K2_VARIANT, the shapes profiles/sweep_env.py compares: CTA-shared tiles of other
-    heights / in place with three buffers, warp-private tiles with 5-12 warps, two or three staging buffers, two to four CTAs
-    per SM, and the 128-point warp-private form) runs the same arithmetic in the same order, so its power maps and detection
-    lists must equal the default form's byte for byte — on a full-length shape, a 128-point shape and a chirp-padded one
-    (130 -> 256 chirps: the PAD instantiations, rows staged at a stride of C elements)."""
+@pytest.mark.parametrize("shape,variants", [((512, 256, 12), ["cube", "split"]), ((256, 128, 4), ["cube", "split"]),
+                                            ((500, 130, 2), ["cube", "split"])])
+def test_doppler_kernel_forms_give_the_same_bits(pkg, shape, variants):
+    """The other forms of K2 run the same arithmetic in the same order as the default one, so the power maps must be equal
+    byte for byte: "cube" keeps the Doppler cube (CTA-shared tiles that also store the cube, where fused mode runs the
+    warp-private kernel at 256 points), "split" is a one-frame batch (the antenna-split path: one single-antenna K2 pass
+    per antenna, then the ordered sum).  The detection list of the split batch equals frame 0's records of the default
+    one byte for byte; cube mode measures its snapshots from the cube, so there cells, powers, noise and flags must match.
+    Shapes: full length, 128 points, and chirp-padded (130 -> 256 chirps: the PAD instantiations)."""
     S, C, A = shape
     F = 5                                                    # several tiles per warp and a ragged tail
     adc = pkg.synth.cube_batch(F, S, C, A, cfg=3, n_targets=6)
-    monkeypatch.delenv("MMW_K2_VARIANT", raising=False)
     with pkg.RadarContext(S, C, A, F) as ctx:
         want, _ = ctx.process_host(adc, F)
         want = want.copy()
         pmaps = [ctx.power_map(f).copy() for f in range(F)]
     assert len(want) > 0
     for v in variants:
-        monkeypatch.setenv("MMW_K2_VARIANT", str(v))
-        with pkg.RadarContext(S, C, A, F) as ctx:
-            got, _ = ctx.process_host(adc, F)
-            for f in range(F):
-                assert np.array_equal(ctx.power_map(f), pmaps[f]), f"K2 variant {v}: power map of frame {f} differs"
-            assert got.tobytes() == want.tobytes(), f"K2 variant {v}: detection list differs"
+        with pkg.RadarContext(S, C, A, F, keep_doppler_cube=(v == "cube")) as ctx:
+            n = F if v == "cube" else 1
+            got, _ = ctx.process_host(adc[:n], n)
+            for f in range(n):
+                assert np.array_equal(ctx.power_map(f), pmaps[f]), f"{v}: power map of frame {f} differs"
+        if v == "split":
+            assert got.tobytes() == want[want["frame"] == 0].tobytes(), "split: detection list differs"
+        else:
+            for fld in ("frame", "range_bin", "doppler_bin", "power", "noise", "flags"):
+                assert np.array_equal(got[fld], want[fld]), f"cube: {fld} differs"
 
 
-@pytest.mark.parametrize("shape,variant", [((512, 256, 12), 5), ((256, 128, 4), 6), ((1024, 64, 2), 6), ((500, 130, 2), 5)])
-def test_range_kernel_forms_give_the_same_bits(pkg, shape, variant, monkeypatch):
-    """The other tile heights of K1 (MMW_K1_VARIANT: 32-row tiles at 512 points, 16-row tiles at 256, 8-row tiles at 1024) and
-    both ways of handing tiles out (MMW_SCHED: counter or fixed stride) compute every chirp's transform with the same
-    arithmetic: range spectra, power maps and lists must equal the default's byte for byte."""
+@pytest.mark.parametrize("shape,F", [((512, 256, 12), 5), ((256, 128, 4), 6), ((1024, 64, 2), 6), ((500, 130, 2), 5)])
+def test_range_kernel_forms_give_the_same_bits(pkg, shape, F, monkeypatch):
+    """Both ways of handing tiles out (MMW_SCHED: counter or fixed stride) compute every chirp's transform with the same
+    arithmetic: range spectra, power maps and lists must equal the default's byte for byte (F frames: several tiles per
+    CTA and a ragged tail)."""
     S, C, A = shape
-    F = 3
     adc = pkg.synth.cube_batch(F, S, C, A, cfg=3, n_targets=6)
-    for name in ("MMW_K1_VARIANT", "MMW_SCHED"):
-        monkeypatch.delenv(name, raising=False)
+    monkeypatch.delenv("MMW_SCHED", raising=False)
     with pkg.RadarContext(S, C, A, F) as ctx:
         want, _ = ctx.process_host(adc, F)
         want = want.copy()
         rs = ctx.range_spectrum(F - 1).copy()
         pm = ctx.power_map(F - 1).copy()
-    for env in ({"MMW_K1_VARIANT": str(variant)}, {"MMW_SCHED": "0"}, {"MMW_SCHED": "3"}):
-        for k, v in env.items():
-            monkeypatch.setenv(k, v)
+    for sched in ("0", "3"):
+        monkeypatch.setenv("MMW_SCHED", sched)
         with pkg.RadarContext(S, C, A, F) as ctx:
             got, _ = ctx.process_host(adc, F)
-            assert np.array_equal(ctx.range_spectrum(F - 1), rs), f"{env}: range spectrum differs"
-            assert np.array_equal(ctx.power_map(F - 1), pm), f"{env}: power map differs"
-            assert got.tobytes() == want.tobytes(), f"{env}: detection list differs"
-        for k in env:
-            monkeypatch.delenv(k)
+            assert np.array_equal(ctx.range_spectrum(F - 1), rs), f"MMW_SCHED={sched}: range spectrum differs"
+            assert np.array_equal(ctx.power_map(F - 1), pm), f"MMW_SCHED={sched}: power map differs"
+            assert got.tobytes() == want.tobytes(), f"MMW_SCHED={sched}: detection list differs"
+        monkeypatch.delenv("MMW_SCHED")
