@@ -335,8 +335,8 @@ int mmw_create(const mmw_config *cfg, mmw_ctx **out)
     if ((rc = dev_alloc(c, &c->d_counts, (size_t)F))) return fail(rc);
     if ((rc = dev_alloc(c, &c->d_offsets, (size_t)F + 1))) return fail(rc);
     if ((rc = dev_alloc(c, &c->d_ticket, (size_t)4))) return fail(rc);
-    if ((rc = dev_alloc(c, &c->d_sched, (size_t)8))) return fail(rc);
-    if (cudaMemset(c->d_sched, 0, 8 * sizeof(unsigned int)) != cudaSuccess) { set_last_error("cudaMemset failed"); return fail(MMW_ERR_CUDA); }
+    if ((rc = dev_alloc(c, &c->d_sched, (size_t)2))) return fail(rc);
+    if (cudaMemset(c->d_sched, 0, 2 * sizeof(unsigned int)) != cudaSuccess) { set_last_error("cudaMemset failed"); return fail(MMW_ERR_CUDA); }
     if (cudaMemset(c->d_ticket, 0, 4 * sizeof(unsigned int)) != cudaSuccess) { set_last_error("cudaMemset failed"); return fail(MMW_ERR_CUDA); }
     c->dense_cap = F * cfg->max_det_per_frame;
     // wide arrays without a Doppler cube: snapshots of the detected cells come from a selective re-FFT of the hit rows
@@ -376,7 +376,6 @@ int mmw_create(const mmw_config *cfg, mmw_ctx **out)
     p.base_adc = nullptr;
     p.sched = c->d_sched;
     p.detect_path = MMW_DETECT_AUTO;
-    p.sched_dynamic = getenv("MMW_SCHED") ? env_int("MMW_SCHED") : 1;
     p.win_r = c->d_win_r; p.win_d = c->d_win_d; p.tw_d = c->d_tw_d; p.tw_a = c->d_tw_a; p.tw1_r = c->d_tw1_r; p.tw1_d = c->d_tw1_d;
 
     // antenna-split Doppler path of small batches (run_front): per-antenna power maps for the largest batch that still

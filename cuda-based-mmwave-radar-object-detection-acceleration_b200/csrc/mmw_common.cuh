@@ -26,14 +26,13 @@ struct PlanDev {
     const float2 *tw1_r;    // [Sp]  pass-1 twiddles of the range FFT in consumption order (tw1_index)
     const float2 *tw1_d;    // [Cp]  pass-1 twiddles of the Doppler FFT in consumption order
     const float2 *tw_a;     // [n_theta]
-    unsigned int *sched;    // [8] work counters of the persistent FFT kernels: {next item, CTAs retired} for K1 at [0], K2 at [2]; zero between launches
+    unsigned int *sched;    // [2] K1's tile counter {next tile, CTAs retired}; zero between launches
     const int16_t *base_adc; // one frame [C][A][S] IIQQ subtracted before the range window, or nullptr (static-clutter removal)
     int detect_path;        // host-side only: MMW_DETECT_AUTO / _PER_CELL / _REFFT (mmw_set_detect_path), read by launch_detect
-    int sched_dynamic;      // bit 0: K1, bit 1: K2 take their tiles from PlanDev.sched instead of a fixed stride (MMW_SCHED; default 1)
     // Padding to a multiple of 16 bytes: the pointer arguments after the plan then keep their 16-byte pairing, which the
     // compiler loads with one 128-bit constant load (measure_wide_kernel).  alignas(16) would do the same but changes
     // the code of the kernels that read the plan's first fields.
-    int pad_[2];
+    int pad_[3];
 };
 static_assert(sizeof(PlanDev) % 16 == 0, "PlanDev size");
 

@@ -15,7 +15,7 @@
 // corner-turned layout directly with fully coalesced stores: the transpose never exists as a
 // separate step and never round-trips HBM.
 //
-// Both kernels are persistent (grid = resident CTAs, each walks a strided list of tiles) and
+// Both kernels are persistent (grid = resident CTAs; K1 takes its tiles from a counter, K2 at a fixed stride) and
 // software-pipelined: the TMA copies of the next tile are issued as soon as the staging buffer
 // of the current one has been consumed, so the copy latency hides behind the second FFT pass.
 #include <stdlib.h>
@@ -41,8 +41,8 @@ void plan_radices(int n, int *r1, int *r2)
     }
 }
 
-// Work counters of the persistent FFT kernels (PlanDev.sched: {next item, CTAs retired} per kernel).  The last CTA to retire puts
-// both back to zero for the next launch on the stream (launches that share a counter pair are stream-ordered).
+// K1's tile counter (PlanDev.sched: {next tile, CTAs retired}).  The last CTA to retire puts both back to zero for the next
+// launch on the stream (launches that share the counter pair are stream-ordered).
 __device__ __forceinline__ void sched_retire(unsigned int *ctr)
 {
     __threadfence();
@@ -124,12 +124,10 @@ __global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, BASE>::kBytes <
     // Tiles are handed out by a counter (PlanDev.sched), not by a fixed stride: a CTA that starts late — its SM was still held by
     // a kernel of another stream (another batch in flight, the exchange's merge kernel) — simply takes fewer tiles instead of
     // finishing its fixed share late.  The first tile of a CTA is blockIdx.x; the next one is fetched while pass 1 runs.
-    const bool DYN = (p.sched_dynamic & 1) != 0;
     __shared__ int s_next[2];
     unsigned int *ctr = p.sched;                                      // [0] next tile - gridDim.x, [1] CTAs done
     if (tid == 0) {
         mbar_init(&bar[0], 1);
-        mbar_init(&bar[1], 1);                                        // not waited on since the double buffer went; kept: same machine code
         fence_mbar_init();
     }
     __syncthreads();
@@ -149,7 +147,7 @@ __global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, BASE>::kBytes <
         const bool row_ok = c0 + row < C;
         const float wdop = row_ok ? p.win_d[c0 + row] : 0.f;
         unsigned int fetched = 0u;
-        if (DYN && tid == 0) fetched = atomicAdd(&ctr[0], 1u);        // answer needed after pass 1 only
+        if (tid == 0) fetched = atomicAdd(&ctr[0], 1u);               // answer needed after pass 1 only
         mbar_wait(&bar[0], (uint32_t)(it & 1));
         const unsigned char *srow = stage + row * L::kStageStride;
         const unsigned char *brow = BASE ? bstage + row * L::kStageStride : nullptr;
@@ -229,9 +227,9 @@ __global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, BASE>::kBytes <
                 }
             }
         }
-        if (DYN && tid == 0) s_next[(it + 1) & 1] = (int)min(fetched + gridDim.x, (unsigned int)n_tiles);
+        if (tid == 0) s_next[(it + 1) & 1] = (int)min(fetched + gridDim.x, (unsigned int)n_tiles);
         __syncthreads();
-        const int next_tile = DYN ? s_next[(it + 1) & 1] : tile + (int)gridDim.x;
+        const int next_tile = s_next[(it + 1) & 1];
         // the staging buffer is consumed now: prefetch the next tile behind pass 2.  (Refilling it earlier — as
         // soon as the last warp has pulled its pass-1 inputs into registers — removes the wait on the copy but not a
         // microsecond of run time: the stall moves to the barrier, profiles/experiments/r1_k1_early_release.md.  L2 prefetch
@@ -260,7 +258,7 @@ __global__ void __launch_bounds__(NW * 32, (2 * RangeSmem<N, BT, BASE>::kBytes <
         __syncthreads();
         tile = next_tile;
     }
-    if (DYN && tid == 0) sched_retire(ctr);
+    if (tid == 0) sched_retire(ctr);
 }
 
 // ---------------------------------------------------------------------------
@@ -336,29 +334,13 @@ __global__ void __launch_bounds__(NW * 32, doppler_min_ctas<N, BT, NW, NSTAGE, I
     const int nrt = Sp / BT;
 
     // a "step" is one antenna of one tile; the q-th step of this CTA is antenna q % A of its (q / A)-th tile, and
-    // steps of consecutive tiles are pipelined back to back
-    // Tiles are handed out by a counter (PlanDev.sched[2], see range_fft_kernel): the CTA's first tile is blockIdx.x, the
-    // tile of ordinal o > 0 is gridDim.x + the counter's value when warp 0 asked.  Warp 0, which issues the staging copies up
-    // to two tiles ahead of the transform, keeps the answers in a four-entry queue in shared memory; its request for the next
-    // ordinal is in flight while the current one is staged, so nobody waits for the atomic.
-    __shared__ int s_tileq[4];
-    unsigned int *ctr = p.sched + 2;
-    const bool dyn = (p.sched_dynamic & 2) != 0;                       // else: the fixed stride gridDim.x
-    unsigned int pending = 0u;                                        // warp 0, lane 0: answer for ordinal `stored`
-    int stored = 1;                                                   // ordinals < stored are in the queue
+    // steps of consecutive tiles are pipelined back to back.  The tile of ordinal o is blockIdx.x + o * gridDim.x: K2 keeps
+    // the fixed stride (K1's counter was slower on cfg3 and cfg5, faster on cfg2: profiles/r2/sweep_tile_scheduling.log).
     auto issue_step = [&](int q) {                                    // warp 0
         const int itq = q / A, a = q - itq * A;
-        if (itq >= stored) {                                          // first step of a new ordinal (they come in order)
-            if (lane == 0) {
-                const unsigned int t = dyn ? pending + gridDim.x : blockIdx.x + (unsigned int)itq * gridDim.x;
-                s_tileq[itq & 3] = (int)(t < (unsigned int)n_tiles ? t : (unsigned int)n_tiles);
-                if (dyn) pending = atomicAdd(&ctr[0], 1u);
-            }
-            ++stored;
-            __syncwarp();
-        }
-        const int tile = s_tileq[itq & 3];
-        if (tile >= n_tiles) return;
+        const unsigned int t = blockIdx.x + (unsigned int)itq * gridDim.x;
+        if (t >= (unsigned int)n_tiles) return;
+        const int tile = (int)t;
         const int rt = tile % nrt, f = tile / nrt;
         const int buf = q % NSTAGE;
         uint64_t *b = &bar[buf];
@@ -379,12 +361,8 @@ __global__ void __launch_bounds__(NW * 32, doppler_min_ctas<N, BT, NW, NSTAGE, I
 #pragma unroll
         for (int i = 0; i < NSTAGE; ++i) mbar_init(&bar[i], 1);
         fence_mbar_init();
-        s_tileq[0] = (int)min(blockIdx.x, (unsigned int)n_tiles);
-        if (dyn) pending = atomicAdd(&ctr[0], 1u);                    // ordinal 1
     }
     __syncthreads();
-    int tile = s_tileq[0];
-    int ord = 0;
     if (warp == 0) {
 #pragma unroll
         for (int i = 0; i < AHEAD; ++i) issue_step(i);
@@ -402,7 +380,7 @@ __global__ void __launch_bounds__(NW * 32, doppler_min_ctas<N, BT, NW, NSTAGE, I
     }
 
 #pragma unroll 1
-    for (; tile < n_tiles; tile = s_tileq[++ord & 3]) {              // (warp 0 queued the next ordinal at least one barrier ago)
+    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const int rt = tile % nrt, f = tile / nrt;
         const int r0 = rt * BT;
         float acc[UPS2][R2];
@@ -479,10 +457,6 @@ __global__ void __launch_bounds__(NW * 32, doppler_min_ctas<N, BT, NW, NSTAGE, I
                 for (int k2 = 0; k2 < R2; ++k2) o[(size_t)(R1 * k2) * Sp] = acc[ui][k2];
             }
         }
-    }
-    if (dyn) {
-        __syncthreads();
-        if (tid == 0) sched_retire(ctr);
     }
 }
 
@@ -725,26 +699,12 @@ __global__ void __launch_bounds__(NW * 32, MINB) doppler_fft_warp_kernel(PlanDev
     const int nrt = Sp / ROWS;
     const long long gw = (long long)blockIdx.x * NW + warp, nwarp = (long long)gridDim.x * NW;
 
-    // Tiles are handed out by a counter (PlanDev.sched[2]): a warp's first tile is its global index, every later one is
-    // nwarp + the counter's value when the warp asked — a warp of a CTA that started late takes fewer tiles.  The staging copies
-    // run NSTAGE - 1 steps ahead, i.e. up to two tiles ahead of the one being transformed, so a warp knows its next two tiles
-    // (t1, t2); the request for the one after is issued when a tile starts and collected when it ends.
-    unsigned int *ctr = p.sched + 2;
-    const bool dyn = (p.sched_dynamic & 2) != 0;                     // else: the fixed stride nwarp
-    auto request = [&]() -> unsigned int { return dyn && lane == 0 ? atomicAdd(&ctr[0], 1u) : 0u; };
-    auto collect = [&](unsigned int r, long long prev) -> long long { return dyn ? nwarp + (long long)__shfl_sync(0xffffffffu, r, 0) : prev + nwarp; };
-    long long t0 = gw, t1, t2;                                      // the tile being transformed and the next two of this warp
-    {
-        const unsigned int r1 = request(), r2 = request();
-        t1 = collect(r1, t0);
-        t2 = collect(r2, t1);
-    }
-
+    // A warp walks the tiles gw, gw + nwarp, gw + 2 nwarp, ...: the fixed stride of doppler_fft_kernel.
     // Staging side.  The ROWS rows of a tile are neighbours in rs ([f][a][Sp][C]), so one step is ONE bulk copy of ROWS * C
     // elements, issued by lane 0: the rows land back to back at the head of the ring slot (row i at i * C), pass 1 pulls them
     // into registers and writes its outputs over them in the padded layout (row i at i * kRowStride).  The step to stage next
-    // is running state — its antenna, its tile (is_d-th after the one being transformed), its ring slot, its source address —
-    // advanced by additions; the only division left is one per tile.
+    // runs NSTAGE - 1 steps ahead of the transform and is running state — its antenna, its tile, its ring slot, its source
+    // address — advanced by additions; the only division left is one per tile.
     const uint32_t step_bytes = (uint32_t)(ROWS * C * 8);
     const size_t ant_stride = (size_t)Sp * C;                       // float2 between the antennas of one (frame, range bin)
     auto tile_src = [&](long long tl) -> const float2 * {
@@ -752,12 +712,12 @@ __global__ void __launch_bounds__(NW * 32, MINB) doppler_fft_warp_kernel(PlanDev
         const int rt = tile % nrt, f = tile / nrt;
         return rs + ((size_t)f * A * Sp + (size_t)rt * ROWS) * (size_t)C;
     };
-    int is_a = 0, is_d = 0, is_slot = 0;                            // is_d: 0, 1 or 2 (the copies run NSTAGE - 1 <= 2 steps ahead)
+    long long is_tile = gw;
+    int is_a = 0, is_slot = 0;
     const float2 *is_src = rs;
     auto issue_next = [&]() {
-        const long long tl = is_d == 0 ? t0 : (is_d == 1 ? t1 : t2);
-        if (tl < n_tiles) {
-            if (is_a == 0) is_src = tile_src(tl);
+        if (is_tile < n_tiles) {
+            if (is_a == 0) is_src = tile_src(is_tile);
             if (lane == 0) {
                 uint64_t *b = &bar[is_slot];
                 fence_proxy_async();
@@ -769,7 +729,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) doppler_fft_warp_kernel(PlanDev
         is_slot = is_slot + 1 == NSTAGE ? 0 : is_slot + 1;
         if (++is_a == A) {
             is_a = 0;
-            ++is_d;
+            is_tile += nwarp;
         }
     };
 
@@ -793,10 +753,9 @@ __global__ void __launch_bounds__(NW * 32, MINB) doppler_fft_warp_kernel(PlanDev
 
     int q = 0;
 #pragma unroll 1
-    while (t0 < n_tiles) {
-        const int tile = (int)t0;
+    for (long long t = gw; t < n_tiles; t += nwarp) {
+        const int tile = (int)t;
         const int rt = tile % nrt, f = tile / nrt;
-        const unsigned int req = request();                         // the tile after t2: collected when this tile ends
         float2 acc[U2][R2 / 2];                                     // bins k2 = 2 j, 2 j + 1
 #pragma unroll
         for (int u = 0; u < U2; ++u)
@@ -860,14 +819,6 @@ __global__ void __launch_bounds__(NW * 32, MINB) doppler_fft_warp_kernel(PlanDev
                 po[(size_t)(k1 + R1 * (2 * j + 1)) * Sp] = acc[u][j].y;
             }
         }
-        t0 = t1;
-        t1 = t2;
-        t2 = collect(req, t2);
-        --is_d;
-    }
-    if (dyn) {
-        __syncthreads();
-        if (tid == 0) sched_retire(ctr);
     }
 }
 
@@ -958,12 +909,24 @@ cudaError_t launch_power_sum(const PlanDev &p, const float *per_antenna, float *
     return cudaGetLastError();
 }
 
-template <typename K>
-static cudaError_t resident_ctas(K kernel, int threads, int smem_bytes, int *ctas_per_sm)
+// Resident CTAs per SM of `Kernel` at `threads` threads and `smem_bytes` of dynamic shared memory, on the current device
+// (which also opts the kernel in to that much shared memory); looked up once per device.  A kernel that cannot be resident
+// at all is an error.
+template <auto Kernel>
+static cudaError_t resident_per_sm(int threads, int smem_bytes, int *per_sm)
 {
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
-    if (e != cudaSuccess) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, kernel, threads, smem_bytes);
+    static int cached[kMaxDevices] = {0};
+    int &n = cached[current_device()];
+    if (!n) {
+        int m = 0;
+        cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
+        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&m, Kernel, threads, smem_bytes);
+        if (e != cudaSuccess) return e;
+        if (m < 1) return cudaErrorLaunchOutOfResources;
+        n = m;
+    }
+    *per_sm = n;
+    return cudaSuccess;
 }
 
 // Grid of a persistent FFT kernel: every resident CTA slot, or fewer when there is less work than that
@@ -976,15 +939,11 @@ static int persistent_grid(int per_sm, long long work_items)
 template <int N, int R1, int R2, int BT, int NW, bool PAIR, bool PAD, int CT, bool BASE = false>
 static cudaError_t run_range_t(const PlanDev &p, const int16_t *adc, float2 *rs, int n_frames, cudaStream_t st)
 {
-    auto k = range_fft_kernel<N, R1, R2, BT, NW, PAIR, PAD, CT, BASE>;
+    constexpr auto k = range_fft_kernel<N, R1, R2, BT, NW, PAIR, PAD, CT, BASE>;
     constexpr int bytes = RangeSmem<N, BT, BASE>::kBytes;
-    static int per_sm_dev[kMaxDevices] = {0};
-    int &per_sm = per_sm_dev[current_device()];
-    if (!per_sm) {
-        cudaError_t e = resident_ctas(k, NW * 32, bytes, &per_sm);
-        if (e != cudaSuccess) return e;
-        if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    }
+    int per_sm = 0;
+    const cudaError_t e = resident_per_sm<k>(NW * 32, bytes, &per_sm);
+    if (e != cudaSuccess) return e;
     const int nct = (p.C + BT - 1) / BT;
     const long long tiles = (long long)n_frames * p.A * nct;
     const int grid = persistent_grid(per_sm, tiles);
@@ -1012,15 +971,11 @@ static cudaError_t run_range(const PlanDev &p, const int16_t *adc, float2 *rs, i
 template <int N, int R1, int R2, int BT, int NW, bool PAD, int SPT, int NSTAGE, bool INPLACE>
 static cudaError_t run_doppler_t(const PlanDev &p, const float2 *rs, float2 *cube, float *pmap, int n_frames, cudaStream_t st)
 {
-    auto k = doppler_fft_kernel<N, R1, R2, BT, NW, PAD, SPT, NSTAGE, INPLACE>;
+    constexpr auto k = doppler_fft_kernel<N, R1, R2, BT, NW, PAD, SPT, NSTAGE, INPLACE>;
     constexpr int bytes = DopplerSmem<N, BT, NSTAGE, INPLACE>::kBytes;
-    static int per_sm_dev[kMaxDevices] = {0};
-    int &per_sm = per_sm_dev[current_device()];
-    if (!per_sm) {
-        cudaError_t e = resident_ctas(k, NW * 32, bytes, &per_sm);
-        if (e != cudaSuccess) return e;
-        if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    }
+    int per_sm = 0;
+    const cudaError_t e = resident_per_sm<k>(NW * 32, bytes, &per_sm);
+    if (e != cudaSuccess) return e;
     const long long tiles = (long long)n_frames * (p.Sp / BT);
     const int grid = persistent_grid(per_sm, tiles);
     k<<<grid, NW * 32, bytes, st>>>(p, rs, cube, pmap, (int)tiles);
@@ -1030,16 +985,12 @@ static cudaError_t run_doppler_t(const PlanDev &p, const float2 *rs, float2 *cub
 template <int N, int R1, int R2, int NW, bool PAD, int SPT, int NSTAGE, int MINB = 2>
 static cudaError_t run_doppler_warp_t(const PlanDev &p, const float2 *rs, float *pmap, int n_frames, cudaStream_t st)
 {
-    auto k = doppler_fft_warp_kernel<N, R1, R2, NW, PAD, SPT, NSTAGE, MINB>;
+    constexpr auto k = doppler_fft_warp_kernel<N, R1, R2, NW, PAD, SPT, NSTAGE, MINB>;
     using L = DopplerWarp<N, R1, R2>;
     constexpr int bytes = L::bytes(NW, NSTAGE);
-    static int per_sm_dev[kMaxDevices] = {0};
-    int &per_sm = per_sm_dev[current_device()];
-    if (!per_sm) {
-        cudaError_t e = resident_ctas(k, NW * 32, bytes, &per_sm);
-        if (e != cudaSuccess) return e;
-        if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    }
+    int per_sm = 0;
+    const cudaError_t e = resident_per_sm<k>(NW * 32, bytes, &per_sm);
+    if (e != cudaSuccess) return e;
     const long long tiles = (long long)n_frames * (p.Sp / L::kRows);
     const long long want = (tiles + NW - 1) / NW;
     const int grid = persistent_grid(per_sm, want);
@@ -1127,20 +1078,15 @@ cudaError_t launch_doppler_fft(const PlanDev &p, const float2 *rs, float2 *cube,
     }
 }
 
-template <int N, int R1, int R2, int BT, int NW>
-static cudaError_t run_extract(const PlanDev &p, const float2 *rs, const uint32_t *keys, const uint32_t *offsets, const uint4 *rows,
-                               const unsigned int *n_rows, float2 *snap, int dense_cap, int max_rows, cudaStream_t st)
+template <int N, int R1, int R2, int BT, int NW, bool PAD>
+static cudaError_t run_extract_t(const PlanDev &p, const float2 *rs, const uint32_t *keys, const uint32_t *offsets, const uint4 *rows,
+                                 const unsigned int *n_rows, float2 *snap, int dense_cap, int max_rows, cudaStream_t st)
 {
+    constexpr auto k = doppler_extract_kernel<N, R1, R2, BT, NW, PAD>;
     constexpr int bytes = ExtractSmem<N, BT>::kBytes;
-    const bool pad = p.C != N;
-    auto k = pad ? doppler_extract_kernel<N, R1, R2, BT, NW, true> : doppler_extract_kernel<N, R1, R2, BT, NW, false>;
-    static int per_sm_dev[kMaxDevices][2] = {{0}};
-    int &per_sm = per_sm_dev[current_device()][pad ? 1 : 0];
-    if (!per_sm) {
-        cudaError_t e = resident_ctas(k, NW * 32, bytes, &per_sm);
-        if (e != cudaSuccess) return e;
-        if (per_sm < 1) return cudaErrorLaunchOutOfResources;
-    }
+    int per_sm = 0;
+    const cudaError_t e = resident_per_sm<k>(NW * 32, bytes, &per_sm);
+    if (e != cudaSuccess) return e;
     // the number of hit rows is only known on the device: a persistent grid of every resident CTA, capped by the most work
     // items there can be (a tile's antennas are split into chunks of >= 4 inside the kernel); idle CTAs leave at once
     const long long items_max = (((long long)max_rows + BT - 1) / BT) * ((p.A + 3) / 4);
@@ -1148,6 +1094,14 @@ static cudaError_t run_extract(const PlanDev &p, const float2 *rs, const uint32_
     const int grid = (int)(items_max < resident ? (items_max < 1 ? 1 : items_max) : resident);
     k<<<grid, NW * 32, bytes, st>>>(p, rs, keys, offsets, rows, n_rows, snap, dense_cap);
     return cudaGetLastError();
+}
+
+template <int N, int R1, int R2, int BT, int NW>
+static cudaError_t run_extract(const PlanDev &p, const float2 *rs, const uint32_t *keys, const uint32_t *offsets, const uint4 *rows,
+                               const unsigned int *n_rows, float2 *snap, int dense_cap, int max_rows, cudaStream_t st)
+{
+    if (p.C == N) return run_extract_t<N, R1, R2, BT, NW, false>(p, rs, keys, offsets, rows, n_rows, snap, dense_cap, max_rows, st);
+    return run_extract_t<N, R1, R2, BT, NW, true>(p, rs, keys, offsets, rows, n_rows, snap, dense_cap, max_rows, st);
 }
 
 // max_rows: upper bound of the hit rows (n_frames * Sp); the true count is read from *n_rows on the device

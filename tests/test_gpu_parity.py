@@ -464,26 +464,3 @@ def test_doppler_kernel_forms_give_the_same_bits(pkg, shape, variants):
         else:
             for fld in ("frame", "range_bin", "doppler_bin", "power", "noise", "flags"):
                 assert np.array_equal(got[fld], want[fld]), f"cube: {fld} differs"
-
-
-@pytest.mark.parametrize("shape,F", [((512, 256, 12), 5), ((256, 128, 4), 6), ((1024, 64, 2), 6), ((500, 130, 2), 5)])
-def test_range_kernel_forms_give_the_same_bits(pkg, shape, F, monkeypatch):
-    """Both ways of handing tiles out (MMW_SCHED: counter or fixed stride) compute every chirp's transform with the same
-    arithmetic: range spectra, power maps and lists must equal the default's byte for byte (F frames: several tiles per
-    CTA and a ragged tail)."""
-    S, C, A = shape
-    adc = pkg.synth.cube_batch(F, S, C, A, cfg=3, n_targets=6)
-    monkeypatch.delenv("MMW_SCHED", raising=False)
-    with pkg.RadarContext(S, C, A, F) as ctx:
-        want, _ = ctx.process_host(adc, F)
-        want = want.copy()
-        rs = ctx.range_spectrum(F - 1).copy()
-        pm = ctx.power_map(F - 1).copy()
-    for sched in ("0", "3"):
-        monkeypatch.setenv("MMW_SCHED", sched)
-        with pkg.RadarContext(S, C, A, F) as ctx:
-            got, _ = ctx.process_host(adc, F)
-            assert np.array_equal(ctx.range_spectrum(F - 1), rs), f"MMW_SCHED={sched}: range spectrum differs"
-            assert np.array_equal(ctx.power_map(F - 1), pm), f"MMW_SCHED={sched}: power map differs"
-            assert got.tobytes() == want.tobytes(), f"MMW_SCHED={sched}: detection list differs"
-        monkeypatch.delenv("MMW_SCHED")
