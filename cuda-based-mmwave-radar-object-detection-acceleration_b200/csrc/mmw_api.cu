@@ -339,10 +339,6 @@ int mmw_create(const mmw_config *cfg, mmw_ctx **out)
     if (cudaMemset(c->d_sched, 0, 2 * sizeof(unsigned int)) != cudaSuccess) { set_last_error("cudaMemset failed"); return fail(MMW_ERR_CUDA); }
     if (cudaMemset(c->d_ticket, 0, 4 * sizeof(unsigned int)) != cudaSuccess) { set_last_error("cudaMemset failed"); return fail(MMW_ERR_CUDA); }
     c->dense_cap = F * cfg->max_det_per_frame;
-    // wide arrays without a Doppler cube: snapshots of the detected cells come from a selective re-FFT of the hit rows
-    // (launch_detect); its buffers scale with the detection capacity — beyond 2 GB the per-detection kernel is used instead.
-    // Narrow arrays get them when the caller picks that path (mmw_set_detect_path).
-    if (A >= 32 && (rc = alloc_refft_buffers(c))) return fail(rc);
     const size_t result_bytes = kResultHeaderBytes + (size_t)c->dense_cap * sizeof(mmw_detection);
     if ((rc = dev_alloc(c, &c->d_result, result_bytes))) return fail(rc);
     c->d_header = reinterpret_cast<uint32_t *>(c->d_result);
@@ -378,6 +374,10 @@ int mmw_create(const mmw_config *cfg, mmw_ctx **out)
     p.detect_path = MMW_DETECT_AUTO;
     p.win_r = c->d_win_r; p.win_d = c->d_win_d; p.tw_d = c->d_tw_d; p.tw_a = c->d_tw_a; p.tw1_r = c->d_tw1_r; p.tw1_d = c->d_tw1_d;
 
+    // buffers of the selective re-FFT path if the plan takes it by default; they scale with the detection capacity — beyond
+    // 2 GB the per-detection kernel is used instead.  Other plans get them when the caller picks that path (mmw_set_detect_path).
+    if (detect_uses_refft(p, true) && (rc = alloc_refft_buffers(c))) return fail(rc);
+
     // antenna-split Doppler path of small batches (run_front): per-antenna power maps for the largest batch that still
     // prefers the split, if that stays modest.  Allocated here, never inside a batch: a batch may be under stream capture.
     if (A > 1 && !cfg->keep_doppler_cube && doppler_prefers_split(p, 1)) {
@@ -402,9 +402,8 @@ int mmw_get_info(const mmw_ctx *c, mmw_info *info)
     const long long N = (long long)p.Sp * p.Cp * p.A, M = (long long)p.Sp * p.Cp;
     info->algorithmic_bytes_per_frame = 28 * N + 8 * M;
     info->workspace_bytes = (long long)c->workspace_bytes;
-    // K1, K2, K3, list, measure; the selective re-FFT path runs rows + extract + angle instead of measure (launch_detect's rule)
-    info->kernels_per_batch = ((p.A >= 32 || p.detect_path == MMW_DETECT_REFFT) && !p.keep_cube && c->d_snap != nullptr &&
-                               p.detect_path != MMW_DETECT_PER_CELL) ? 7 : 5;
+    // K1, K2, K3, list, measure; the selective re-FFT path runs rows + extract + angle instead of measure
+    info->kernels_per_batch = detect_uses_refft(p, c->d_rows != nullptr && c->d_snap != nullptr) ? 7 : 5;
     return MMW_OK;
 }
 

@@ -116,12 +116,14 @@ struct DetectBuffers {
     uint32_t *header;       // {n_written, n_total, n_frames, overflow}
     unsigned int *ticket;   // [0] last-CTA-done counter of list_kernel, [1] work cursor of measure_kernel, [2] hit-row count (all self-resetting)
     mmw_detection *dense;   // ordered detection list of the batch
-    // wide arrays in fused mode (A >= 32, no Doppler cube): the selective Doppler re-FFT path (nullptr: measure_wide_kernel instead)
+    // buffers of the selective Doppler re-FFT path (detect_uses_refft; nullptr: a per-detection kernel instead)
     uint4 *rows;            // [F * Sp] {frame, range bin, dense index of the row's first hit, -}: every (frame, range bin) with hits
     float2 *snap;           // [dense capacity][A] antenna snapshots of the detected cells
 };
 cudaError_t launch_cfar(const PlanDev &p, const float *pmap, uint32_t *mask, float *noise_map, int n_frames, int sm_count, cudaStream_t st);
 cudaError_t launch_detect(const PlanDev &p, const DetectBuffers &b, int n_frames, int dense_cap, int sm_count, cudaStream_t st);
+// whether launch_detect takes the selective re-FFT path for this plan (mmw_detect.cu)
+bool detect_uses_refft(const PlanDev &p, bool have_refft_buffers);
 // the kernels that write mmw_detection records (the only readers of PlanDev.frame_offset, their argument 0): graph mode patches
 // that argument in place instead of re-capturing when the frame offset changes (mmw_api.cu).  Returns the kernel's argument
 // count, 0 if `func` is not one of them.

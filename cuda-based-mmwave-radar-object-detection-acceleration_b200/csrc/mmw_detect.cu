@@ -460,7 +460,9 @@ constexpr int kMeasNT = 256;
 constexpr int kMeasWarps = kMeasNT / 32;
 constexpr int kMeasG = 4;            // detections measured together (they share every range-spectrum row they read)
 constexpr int kMeasQ = 2;            // antennas whose rows are in flight together
-constexpr int kMeasWideA = 32;       // from this many antennas on, a whole CTA (not one warp) measures a chunk ...
+// Wide arrays, from this many antennas on: fused mode takes the selective re-FFT path (detect_uses_refft); otherwise a whole
+// CTA (not one warp) measures a chunk ...
+constexpr int kMeasWideA = 32;
 constexpr int kMeasWideG = 32;       // ... of up to this many detections (kMeasG at a time in registers, rows re-read from L1)
 
 __device__ __forceinline__ float warp_sum(float v)
@@ -497,8 +499,23 @@ __device__ __forceinline__ void lookup_frame(const uint32_t *__restrict__ offset
     fc.fend_raw = offsets[lo + 1];
 }
 
-// Warp-collective.  Returns false if list position g0 is not the head of a chunk.  The neighbouring keys are read 32 at
-// a time, one per lane, so that finding the run costs one memory round trip instead of one per element.
+// Warp-collective: how many list positions directly before g (down to the frame's first, fbeg) have range bin r, i.e. the
+// position of g inside its run of equal range bin.  kf[q] = key of list position q.  The predecessors are read 32 at a
+// time, one per lane, so that finding the run costs one memory round trip instead of one per element.
+__device__ __forceinline__ uint32_t run_back(const uint32_t *__restrict__ kf, uint32_t fbeg, uint32_t g, int r, int lane)
+{
+    uint32_t back = 0;
+    for (uint32_t base = g;;) {
+        const bool same = base >= fbeg + 1 + lane && (int)(kf[base - 1 - lane] >> 16) == r;
+        const uint32_t m = __ballot_sync(0xffffffffu, same);
+        const uint32_t n = m == 0xffffffffu ? 32u : (uint32_t)(__ffs(~m) - 1);
+        back += n;
+        if (n < 32u) return back;
+        base -= 32u;
+    }
+}
+
+// Warp-collective.  Returns false if list position g0 is not the head of a chunk.
 template <int G>
 __device__ __forceinline__ bool locate_chunk(const PlanDev &p, const uint32_t *__restrict__ keys, const uint32_t *__restrict__ offsets,
                                              int n_frames, uint32_t total, uint32_t g0, int lane, MeasFrame &fc, MeasChunk &ch)
@@ -507,16 +524,7 @@ __device__ __forceinline__ bool locate_chunk(const PlanDev &p, const uint32_t *_
     const uint32_t fbeg = fc.fbeg, fend = min(fc.fend_raw, total);
     const uint32_t *kf = keys + (size_t)fc.f * p.max_det - fbeg;  // kf[g] = key of list position g
     const int r = (int)(kf[g0] >> 16);
-    uint32_t back = 0;                                            // position of g0 inside its run of equal range bin
-    for (uint32_t base = g0;;) {                                  // 32 predecessors per round
-        const bool same = base >= fbeg + 1 + lane && (int)(kf[base - 1 - lane] >> 16) == r;
-        const uint32_t m = __ballot_sync(0xffffffffu, same);
-        const uint32_t n = m == 0xffffffffu ? 32u : (uint32_t)(__ffs(~m) - 1);
-        back += n;
-        if (n < 32u) break;
-        base -= 32u;
-    }
-    if (back % G != 0) return false;                              // every G-th detection of a run heads a chunk
+    if (run_back(kf, fbeg, g0, r, lane) % G != 0) return false;   // every G-th detection of a run heads a chunk
     const uint32_t mykey = g0 + lane < fend ? kf[g0 + lane] : 0xffffffffu;      // lane j: key of list position g0 + j
     const uint32_t fm = __ballot_sync(0xffffffffu, g0 + lane < fend && (int)(mykey >> 16) == r);
     ch.f = fc.f;
@@ -603,26 +611,40 @@ __device__ __forceinline__ void snapshot_antennas(const PlanDev &p, const float2
     }
 }
 
-// Warp-collective: strict 3x3 maximum among detected cells (Doppler wraps, range clamps; ties -> lowest (r,d))
-__device__ __forceinline__ bool group_peak(const PlanDev &p, const float *__restrict__ pf, const uint32_t *__restrict__ mf, int r, int d,
-                                           float pw, int lane)
+// The 3x3 grouping test of every detection path: is neighbour `cell` (0..8, row-major over range offsets -1..1 x Doppler
+// offsets -1..1; 4 is the detection itself) of detection (r, d) with power pw a detected cell that outranks it?  Doppler
+// wraps, range clamps; larger power outranks, equal power -> the lower (r, d).  A detection is a peak (strict 3x3 maximum)
+// when none of its eight neighbours outranks it.  pf / mf: the frame's power map and CFAR mask.
+__device__ __forceinline__ bool neighbour_outranks(const PlanDev &p, const float *__restrict__ pf, const uint32_t *__restrict__ mf,
+                                                   int r, int d, float pw, int cell)
 {
     const int Sp = p.Sp, Cp = p.Cp;
-    const uint32_t key = ((uint32_t)r << 16) | (uint32_t)d;
-    bool worse = false;
-    if (lane < 9 && lane != 4) {
-        const int rr = r + lane / 3 - 1;
-        const int dd = (d + lane % 3 - 1 + Cp) & (Cp - 1);
-        if (rr >= 0 && rr < Sp) {
-            const uint32_t w = mf[(size_t)(dd >> 5) * Sp + rr];
-            if ((w >> (dd & 31)) & 1u) {
-                const float pn = pf[(size_t)dd * Sp + rr];
-                const uint32_t kn = ((uint32_t)rr << 16) | (uint32_t)dd;
-                worse = (pn > pw) || (pn == pw && kn < key);
-            }
-        }
+    const int rr = r + cell / 3 - 1;
+    const int dd = (d + cell % 3 - 1 + Cp) & (Cp - 1);
+    if (rr < 0 || rr >= Sp) return false;
+    const uint32_t w = mf[(size_t)(dd >> 5) * Sp + rr];
+    if (!((w >> (dd & 31)) & 1u)) return false;
+    const float pn = pf[(size_t)dd * Sp + rr];
+    const uint32_t key = ((uint32_t)r << 16) | (uint32_t)d, kn = ((uint32_t)rr << 16) | (uint32_t)dd;
+    return (pn > pw) || (pn == pw && kn < key);
+}
+
+// The arg-max tie rule of the angle spectrum: larger power wins, equal power -> lower bin (strict >, first wins).
+__device__ __forceinline__ void argmax_update(float m, int k, float &best, int &bestk)
+{
+    if (m > best || (m == best && k < bestk)) { best = m; bestk = k; }
+}
+
+// Arg-max over aligned groups of WIDTH lanes (xor butterfly); every lane of a group ends with the group's result.
+template <int WIDTH = 32>
+__device__ __forceinline__ void warp_argmax(float &best, int &bestk)
+{
+#pragma unroll
+    for (int o = WIDTH / 2; o > 0; o >>= 1) {
+        const float ob = __shfl_xor_sync(0xffffffffu, best, o);
+        const int ok = __shfl_xor_sync(0xffffffffu, bestk, o);
+        argmax_update(ob, ok, best, bestk);
     }
-    return __ballot_sync(0xffffffffu, worse) == 0u;
 }
 
 __device__ __forceinline__ void angle_bin_power(const float2 *xj, const float2 *twa, int A, int n_theta, int k, float &best, int &bestk)
@@ -634,18 +656,7 @@ __device__ __forceinline__ void angle_bin_power(const float2 *xj, const float2 *
         yx += v.x * w.x - v.y * w.y;
         yy += v.x * w.y + v.y * w.x;
     }
-    const float m = yx * yx + yy * yy;
-    if (m > best || (m == best && k < bestk)) { best = m; bestk = k; }      // strict >, first wins
-}
-
-__device__ __forceinline__ void warp_argmax(float &best, int &bestk)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-        const int ok = __shfl_xor_sync(0xffffffffu, bestk, o);
-        if (ob > best || (ob == best && ok < bestk)) { best = ob; bestk = ok; }
-    }
+    argmax_update(yx * yx + yy * yy, k, best, bestk);
 }
 
 __device__ __forceinline__ void write_record(const PlanDev &p, mmw_detection *__restrict__ dense, uint32_t g, int f, int r, int d, float pw,
@@ -679,22 +690,9 @@ __device__ __forceinline__ void emit_chunk(const PlanDev &p, const float *__rest
     const bool active = j < ch.ng;
     const int r = ch.r;
     const int d = (int)(__shfl_sync(0xffffffffu, ch.mykey, min(j, ch.ng - 1)) & 0xffffu);
-    const uint32_t key = ((uint32_t)r << 16) | (uint32_t)d;
     const float pw = active ? pf[(size_t)d * Sp + r] : 0.f;
     const float noise = (active && nb == 0) ? noise_map[((size_t)ch.f * Cp + d) * Sp + r] : 0.f;
-    // 3x3 grouping among detected cells (Doppler wraps, range clamps; ties -> lowest (r,d)); nb skips the centre
-    const int cell = nb < 4 ? nb : nb + 1;
-    const int rr = r + cell / 3 - 1;
-    const int dd = (d + cell % 3 - 1 + Cp) & (Cp - 1);
-    bool worse = false;
-    if (active && rr >= 0 && rr < Sp) {
-        const uint32_t w = mf[(size_t)(dd >> 5) * Sp + rr];
-        if ((w >> (dd & 31)) & 1u) {
-            const float pn = pf[(size_t)dd * Sp + rr];
-            const uint32_t kn = ((uint32_t)rr << 16) | (uint32_t)dd;
-            worse = (pn > pw) || (pn == pw && kn < key);
-        }
-    }
+    const bool worse = active && neighbour_outranks(p, pf, mf, r, d, pw, nb < 4 ? nb : nb + 1);     // nb skips the centre
     const uint32_t wm = __ballot_sync(0xffffffffu, worse);
     const bool is_peak = ((wm >> (8 * j)) & 0xffu) == 0u;
     int my_bestk = 0;
@@ -750,16 +748,7 @@ __global__ void __launch_bounds__(kMeasNT) measure_kernel(PlanDev p, const float
             const bool valid = g + lane < fend;
             const uint32_t mykey = valid ? kf[g + lane] : 0xffffffffu;
             const int myr = (int)(mykey >> 16);
-            const int r_first = __shfl_sync(0xffffffffu, myr, 0);
-            uint32_t back = 0;                                        // how far the run of position g reaches back
-            for (uint32_t base = g;;) {
-                const bool same = base >= fbeg + 1 + lane && (int)(kf[base - 1 - lane] >> 16) == r_first;
-                const uint32_t m = __ballot_sync(0xffffffffu, same);
-                const uint32_t n = m == 0xffffffffu ? 32u : (uint32_t)(__ffs(~m) - 1);
-                back += n;
-                if (n < 32u) break;
-                base -= 32u;
-            }
+            const uint32_t back = run_back(kf, fbeg, g, __shfl_sync(0xffffffffu, myr, 0), lane);   // how far the run of g reaches back
             // index of every position inside its run of equal range bin -> chunk heads (every kMeasG-th)
             const int prev_r = __shfl_up_sync(0xffffffffu, myr, 1);
             const uint32_t starts = __ballot_sync(0xffffffffu, lane > 0 && valid && myr != prev_r);
@@ -835,7 +824,8 @@ __global__ void __launch_bounds__(kMeasNT) measure_wide_kernel(PlanDev p, const 
                 const int d = ch.doppler(j);
                 const float pw = pf[(size_t)d * Sp + ch.r];
                 const float noise = noise_map[((size_t)ch.f * Cp + d) * Sp + ch.r];
-                const bool is_peak = group_peak(p, pf, mf, ch.r, d, pw, lane);
+                const bool worse = lane < 9 && lane != 4 && neighbour_outranks(p, pf, mf, ch.r, d, pw, lane);
+                const bool is_peak = __ballot_sync(0xffffffffu, worse) == 0u;
                 if (lane == 0) write_record(p, dense, g0 + j, ch.f, ch.r, d, pw, noise, bestk, is_peak);
             }
             __syncthreads();
@@ -944,19 +934,12 @@ __global__ void __launch_bounds__(256) angle_fft_kernel(PlanDev p, const float2 
 #pragma unroll
             for (int k2 = 0; k2 < R2; ++k2) {
                 const float2 v = y[bitrev(k2, LR2)];
-                const float m = v.x * v.x + v.y * v.y;
-                const int k = k1 + R1 * k2;
-                if (m > best || (m == best && k < bestk)) { best = m; bestk = k; }
+                argmax_update(v.x * v.x + v.y * v.y, k1 + R1 * k2, best, bestk);
             }
         }
-#pragma unroll
-        for (int o = SUBS / 2; o > 0; o >>= 1) {
-            const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-            const int ok = __shfl_xor_sync(0xffffffffu, bestk, o);
-            if (ob > best || (ob == best && ok < bestk)) { best = ob; bestk = ok; }
-        }
+        warp_argmax<SUBS>(best, bestk);
         __syncwarp();                                                // the row is free for the next detection
-        // record: lanes 0..7 of the group look at the eight 3x3 neighbours (Doppler wraps, range clamps; ties -> lowest (r, d))
+        // record: lanes 0..7 of the group look at the eight 3x3 neighbours
         bool worse = false;
         int f = 0, rb = 0, d = 0;
         float pw = 0.f, noise = 0.f;
@@ -969,19 +952,7 @@ __global__ void __launch_bounds__(256) angle_fft_kernel(PlanDev p, const float2 
             const float *pf = pmap + (size_t)f * Cp * Sp;
             pw = pf[(size_t)d * Sp + rb];
             if (sub == 0) noise = noise_map[((size_t)f * Cp + d) * Sp + rb];
-            if (sub < 8) {
-                const int cell = sub < 4 ? sub : sub + 1;
-                const int rr = rb + cell / 3 - 1;
-                const int dd = (d + cell % 3 - 1 + Cp) & (Cp - 1);
-                if (rr >= 0 && rr < Sp) {
-                    const uint32_t w = mask[((size_t)f * (Cp / 32) + (dd >> 5)) * Sp + rr];
-                    if ((w >> (dd & 31)) & 1u) {
-                        const float pn = pf[(size_t)dd * Sp + rr];
-                        const uint32_t kn = ((uint32_t)rr << 16) | (uint32_t)dd;
-                        worse = (pn > pw) || (pn == pw && kn < key);
-                    }
-                }
-            }
+            if (sub < 8) worse = neighbour_outranks(p, pf, mask + (size_t)f * (Cp / 32) * Sp, rb, d, pw, sub < 4 ? sub : sub + 1);
         }
         const uint32_t wm = __ballot_sync(0xffffffffu, worse);
         const bool is_peak = ((wm >> (row * SUBS)) & 0xffu) == 0u;
@@ -1097,6 +1068,16 @@ int record_kernel_args(const void *func)
     return 0;
 }
 
+// Wide arrays in fused mode take the selective re-FFT path (rows_kernel -> doppler_extract_kernel -> angle_fft_kernel);
+// everything else takes a per-detection kernel.  PlanDev.detect_path (mmw_set_detect_path) forces either path.  Cube mode
+// has no range spectrum to re-transform and always measures per detection, and so does a context without the re-FFT
+// buffers (have_refft_buffers: rows and snap allocated).
+bool detect_uses_refft(const PlanDev &p, bool have_refft_buffers)
+{
+    if (p.keep_cube || !have_refft_buffers || p.detect_path == MMW_DETECT_PER_CELL) return false;
+    return p.A >= kMeasWideA || p.detect_path == MMW_DETECT_REFFT;
+}
+
 cudaError_t launch_detect(const PlanDev &p, const DetectBuffers &b, int n_frames, int dense_cap, int sm_count, cudaStream_t st)
 {
     const int nwords = p.Sp * p.Cp / 32;
@@ -1112,11 +1093,8 @@ cudaError_t launch_detect(const PlanDev &p, const DetectBuffers &b, int n_frames
     list_kernel<<<n_frames, kListNT, list_bytes, st>>>(p, b.mask, b.keys, b.counts, b.offsets, b.header, b.ticket, n_frames, dense_cap);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    const bool wide = p.A >= kMeasWideA;
-    // wide arrays, fused mode: one more Doppler FFT of the rows that have hits, then the angle spectra as FFTs
-    // (PlanDev.detect_path, mmw_set_detect_path, forces either path)
-    if ((wide || p.detect_path == MMW_DETECT_REFFT) && !p.keep_cube && b.rows != nullptr && b.snap != nullptr &&
-        p.detect_path != MMW_DETECT_PER_CELL) {
+    // re-FFT path: one more Doppler FFT of the rows that have hits, then the angle spectra as FFTs
+    if (detect_uses_refft(p, b.rows != nullptr && b.snap != nullptr)) {
         const int rgrid = (dense_cap + 255) / 256 < sm_count * 4 ? (dense_cap + 255) / 256 : sm_count * 4;
         rows_kernel<<<rgrid < 1 ? 1 : rgrid, 256, 0, st>>>(p, b.keys, b.offsets, b.rows, b.ticket + 2, n_frames, dense_cap);
         e = cudaGetLastError();
@@ -1130,6 +1108,7 @@ cudaError_t launch_detect(const PlanDev &p, const DetectBuffers &b, int n_frames
         default:  return cudaErrorInvalidValue;
         }
     }
+    const bool wide = p.A >= kMeasWideA;
     const int bytes = p.n_theta * 8 + (wide ? kMeasWideG : kMeasWarps * kMeasG) * p.A * 8;
     static int configured_dev[kMaxDevices][2] = {{0}};
     int *configured = configured_dev[current_device()];

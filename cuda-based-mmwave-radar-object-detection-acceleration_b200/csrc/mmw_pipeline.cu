@@ -304,6 +304,52 @@ constexpr int doppler_min_ctas()
     return m < 1 ? 1 : (m > 3 ? 3 : m);
 }
 
+// The two passes of a CTA-shared Doppler tile, shared by doppler_fft_kernel and doppler_extract_kernel so that K2x's
+// snapshots are the very values K2 computes.  A slot (the lanes of a warp that work on one row) owns the butterflies
+// slot, slot + NSLOT, ... of each pass.
+// Pass 1: R2 butterflies of radix R1 over stride R2 (Doppler window already applied by K1), read from srow and written to
+// wrow, which may be srow (a thread reads and writes the same R1 addresses).  TWREG: the slot's twiddles are held in twr;
+// otherwise they are read from tw.  The butterfly's registers x are the caller's, and the zero-fill of padded chirps is
+// written per component: with an array of the helper's own or one float2 select, ptxas allocates doppler_fft_kernel's
+// registers differently from the form the sweeps under profiles/ measured.
+template <int R1, int R2, int NSLOT, bool PAD, bool TWREG>
+__device__ __forceinline__ void doppler_pass1(const float2 *srow, float2 *wrow, const float2 *tw, const float2 (*twr)[TWREG ? R1 - 1 : 1],
+                                              int slot, int C, float2 (&x)[R1])
+{
+    constexpr int LR1 = ilog2(R1);
+    constexpr int UPS1 = (R2 + NSLOT - 1) / NSLOT;
+#pragma unroll
+    for (int ui = 0; ui < UPS1; ++ui) {
+        const int n2 = slot + ui * NSLOT;
+        if (UPS1 * NSLOT == R2 || n2 < R2) {
+#pragma unroll
+            for (int m = 0; m < R1; ++m) {
+                const int n = n2 + m * R2;
+                float vy = 0.f, vx = 0.f;
+                if (!PAD || n < C) { const float2 t = srow[n]; vy = t.y; vx = t.x; }
+                x[m] = make_float2(vx, vy);
+            }
+            dft_regs<R1>(x);
+            float2 *wo = wrow + n2;
+            wo[0] = x[0];
+#pragma unroll
+            for (int k1 = 1; k1 < R1; ++k1) {
+                const float2 w = TWREG ? twr[ui][k1 - 1] : tw[tw1_index(n2, k1, R1)];
+                wo[k1 * R2] = cmul(x[bitrev(k1, LR1)], w);
+            }
+        }
+    }
+}
+
+// Pass 2 of one run: radix R2 on the R2 contiguous pass-1 outputs at wi; bin k1 + R1 * k2 lands in y[bitrev(k2)].
+template <int R2>
+__device__ __forceinline__ void doppler_pass2(const float2 *wi, float2 (&y)[R2])
+{
+#pragma unroll
+    for (int n2 = 0; n2 < R2; ++n2) y[n2] = wi[n2];
+    dft_regs<R2>(y);
+}
+
 template <int N, int R1, int R2, int BT, int NW, bool PAD, int SPT, int NSTAGE, bool INPLACE>
 __global__ void __launch_bounds__(NW * 32, doppler_min_ctas<N, BT, NW, NSTAGE, INPLACE>()) doppler_fft_kernel(PlanDev p, const float2 *__restrict__ rs, float2 *__restrict__ cube,
                                                                float *__restrict__ pmap, int n_tiles)
@@ -315,7 +361,7 @@ __global__ void __launch_bounds__(NW * 32, doppler_min_ctas<N, BT, NW, NSTAGE, I
     constexpr int NT = NW * 32;
     constexpr int SUBS = 32 / BT;
     constexpr int NSLOT = NW * SUBS;
-    constexpr int LR1 = ilog2(R1), LR2 = ilog2(R2);
+    constexpr int LR2 = ilog2(R2);
     constexpr int UPS2 = (R1 + NSLOT - 1) / NSLOT;                   // pass-2 butterflies per slot
     constexpr int UPS1 = (R2 + NSLOT - 1) / NSLOT;                   // pass-1 butterflies per slot
     // a slot's pass-1 butterflies are the same for every step, so their twiddles can live in registers
@@ -398,27 +444,8 @@ __global__ void __launch_bounds__(NW * 32, doppler_min_ctas<N, BT, NW, NSTAGE, I
             float2 *srow = stage + (size_t)(s % NSTAGE) * (BT * L::kStageRow) + row * L::kStageRow;
             float2 *wrow = INPLACE ? srow : work + row * (N + 1);
 
-            // pass 1: R2 butterflies of radix R1 over stride R2 (Doppler window already applied by K1)
-#pragma unroll
-            for (int ui = 0; ui < UPS1; ++ui) {
-                const int n2 = slot + ui * NSLOT;
-                if (UPS1 * NSLOT == R2 || n2 < R2) {
-                    float2 x[R1];
-#pragma unroll
-                    for (int m = 0; m < R1; ++m) {
-                        const int n = n2 + m * R2;
-                        x[m] = (!PAD || n < C) ? srow[n] : make_float2(0.f, 0.f);
-                    }
-                    dft_regs<R1>(x);
-                    float2 *wo = wrow + n2;
-                    wo[0] = x[0];
-#pragma unroll
-                    for (int k1 = 1; k1 < R1; ++k1) {
-                        const float2 w = TWREG ? twr[ui][k1 - 1] : tw[tw1_index(n2, k1, R1)];
-                        wo[k1 * R2] = cmul(x[bitrev(k1, LR1)], w);
-                    }
-                }
-            }
+            float2 x[R1];
+            doppler_pass1<R1, R2, NSLOT, PAD, TWREG>(srow, wrow, tw, twr, slot, C, x);
             __syncthreads();
             if (!INPLACE && NSTAGE == 1 && warp == 0) issue_step(s + 1);   // staging buffer consumed: refill behind pass 2
 
@@ -428,10 +455,7 @@ __global__ void __launch_bounds__(NW * 32, doppler_min_ctas<N, BT, NW, NSTAGE, I
                 const int k1 = slot + ui * NSLOT;
                 if (k1 < R1) {
                     float2 y[R2];
-                    const float2 *wi = wrow + k1 * R2;
-#pragma unroll
-                    for (int n2 = 0; n2 < R2; ++n2) y[n2] = wi[n2];
-                    dft_regs<R2>(y);
+                    doppler_pass2<R2>(wrow + k1 * R2, y);
 #pragma unroll
                     for (int k2 = 0; k2 < R2; ++k2) {
                         const float2 v = y[bitrev(k2, LR2)];
@@ -467,11 +491,11 @@ __global__ void __launch_bounds__(NW * 32, doppler_min_ctas<N, BT, NW, NSTAGE, I
 // Doppler bin d of all A antennas at range bin r.  A direct DFT per detection costs A * C complex MACs and a pass over the
 // A x C block of the range spectrum; on the imaging cube (A = 192, C = 512: 786 KB per range bin) with thousands of hits
 // that was the longest stage of the chain.  Here every (frame, range bin) that has at least one hit — `rows`, made by
-// rows_kernel from the ordered key list — is transformed ONCE more with the very FFT K2 runs (same code, same roundings:
-// the snapshot is bit-identical to what the Doppler cube would hold), and only the detected bins are written out, to
-// snap[dense index][antenna].  Cost: one K2 step per hit row, whatever the number of hits in it — bounded by one K2 pass.
-// A tile is BT arbitrary hit rows (each row is its own bulk copy, so they need not be neighbours); staging, the in-place
-// two-pass FFT and the three-stage ring are doppler_fft_kernel's.
+// rows_kernel from the ordered key list — is transformed ONCE more with the very FFT K2 runs (doppler_pass1 and
+// doppler_pass2: the snapshot is bit-identical to what the Doppler cube would hold), and only the detected bins are written
+// out, to snap[dense index][antenna].  Cost: one K2 step per hit row, whatever the number of hits in it — bounded by one K2
+// pass.  A tile is BT arbitrary hit rows (each row is its own bulk copy, so they need not be neighbours); staging, the
+// in-place pass 1 and the three-stage ring are those of doppler_fft_kernel<.., INPLACE>.
 template <int N, int BT>
 struct ExtractSmem {
     static constexpr int kStageRow = N + 2;
@@ -493,9 +517,8 @@ __global__ void __launch_bounds__(NW * 32, (2 * ExtractSmem<N, BT>::kBytes <= 22
     constexpr int NSTAGE = L::kNStage, AHEAD = NSTAGE - 1;
     constexpr int SUBS = 32 / BT;
     constexpr int NSLOT = NW * SUBS;
-    constexpr int LR1 = ilog2(R1), LR2 = ilog2(R2);
+    constexpr int LR2 = ilog2(R2);
     constexpr int UPS2 = (R1 + NSLOT - 1) / NSLOT;
-    constexpr int UPS1 = (R2 + NSLOT - 1) / NSLOT;
 
     extern __shared__ __align__(16) unsigned char smem[];
     uint64_t *bar = reinterpret_cast<uint64_t *>(smem);
@@ -604,24 +627,8 @@ __global__ void __launch_bounds__(NW * 32, (2 * ExtractSmem<N, BT>::kBytes <= 22
             float2 *sbuf = stage + (size_t)(s % NSTAGE) * (BT * L::kStageRow);
             float2 *srow = sbuf + row * L::kStageRow;
 
-            // pass 1, in place (as doppler_fft_kernel<.., INPLACE>)
-#pragma unroll
-            for (int ui = 0; ui < UPS1; ++ui) {
-                const int n2 = slot + ui * NSLOT;
-                if (UPS1 * NSLOT == R2 || n2 < R2) {
-                    float2 x[R1];
-#pragma unroll
-                    for (int m = 0; m < R1; ++m) {
-                        const int n = n2 + m * R2;
-                        x[m] = (!PAD || n < C) ? srow[n] : make_float2(0.f, 0.f);
-                    }
-                    dft_regs<R1>(x);
-                    float2 *wo = srow + n2;
-                    wo[0] = x[0];
-#pragma unroll
-                    for (int k1 = 1; k1 < R1; ++k1) wo[k1 * R2] = cmul(x[bitrev(k1, LR1)], tw[tw1_index(n2, k1, R1)]);
-                }
-            }
+            float2 x[R1];
+            doppler_pass1<R1, R2, NSLOT, PAD, false>(srow, srow, tw, nullptr, slot, C, x);      // in place
             __syncthreads();
             // pass 2; bin k1 + R1 * k2 goes back to srow[k1 * R2 + k2] (the run this thread has just read)
 #pragma unroll
@@ -630,9 +637,7 @@ __global__ void __launch_bounds__(NW * 32, (2 * ExtractSmem<N, BT>::kBytes <= 22
                 if (k1 < R1) {
                     float2 y[R2];
                     float2 *wi = srow + k1 * R2;
-#pragma unroll
-                    for (int n2 = 0; n2 < R2; ++n2) y[n2] = wi[n2];
-                    dft_regs<R2>(y);
+                    doppler_pass2<R2>(wi, y);
 #pragma unroll
                     for (int k2 = 0; k2 < R2; ++k2) wi[k2] = y[bitrev(k2, LR2)];
                 }
