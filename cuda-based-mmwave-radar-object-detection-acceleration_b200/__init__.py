@@ -9,4 +9,4 @@ The directory name contains hyphens (it mirrors the reference repository's name)
 through `__graft_entry__.load_package()` or importlib, not with an `import` statement.
 """
 from . import api, build, sharding, synth  # noqa: F401
-from .api import DET_DTYPE, TARGET_DTYPE, PeerExchange, RadarContext, RadarError, RadarGroup, RadarParams, cudaProcessing  # noqa: F401
+from .api import DET_DTYPE, OBJ_DTYPE, TARGET_DTYPE, PeerExchange, RadarContext, RadarError, RadarGroup, RadarParams, cudaProcessing  # noqa: F401

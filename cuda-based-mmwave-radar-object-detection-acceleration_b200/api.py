@@ -47,9 +47,32 @@ C_ABI_SYMBOLS = [
     "mmw_group_process_host", "mmw_group_process_device", "mmw_group_merged_block", "mmw_group_read_detections",
     "mmw_exchange_create", "mmw_exchange_destroy", "mmw_exchange_handle", "mmw_exchange_connect", "mmw_exchange_put", "mmw_exchange_merge",
     "mmw_exchange_wait",
+    "mmw_default_cluster_params", "mmw_set_clustering", "mmw_read_objects", "mmw_read_labels", "mmw_device_objects",
+    "mmw_objects_to_physical",
 ]
 # the reference's own entry point (acceleration.h:32), C++ linkage
 LEGACY_MANGLED = "_Z14cudaProcessingPsP9Complex_tiPdS2_S2_S2_"
+
+
+# mmw_object of include/mmw_radar.h (48 bytes); tests/test_cluster_reference.py checks the offsets against the header
+OBJ_DTYPE = np.dtype(
+    [
+        ("frame", "<u4"), ("first_det", "<u4"), ("n_det", "<u4"), ("peak_det", "<u4"),
+        ("range_bin", "<f4"), ("doppler_bin", "<f4"), ("angle_rad", "<f4"),
+        ("power", "<f4"), ("peak_power", "<f4"), ("peak_noise", "<f4"),
+        ("range_min", "<u2"), ("range_max", "<u2"), ("doppler_min", "<i2"), ("doppler_max", "<i2"),
+    ]
+)
+assert OBJ_DTYPE.itemsize == 48
+assert [OBJ_DTYPE.fields[n][1] for n in OBJ_DTYPE.names] == [0, 4, 8, 12, 16, 20, 24, 28, 32, 36, 40, 42, 44, 46]
+OBJECT_HEADER_BYTES = 32
+OBJECTS_CUT, OBJECTS_DETECTIONS_TRUNCATED = 0x1, 0x2       # flag bits of the object header's word 3
+
+
+class ClusterParams(C.Structure):
+    """mmw_cluster_params"""
+    _fields_ = [("eps_range", C.c_int), ("eps_doppler", C.c_int), ("eps_angle", C.c_int), ("min_points", C.c_int),
+                ("max_objects_per_frame", C.c_int)]
 
 
 class Config(C.Structure):
@@ -145,6 +168,13 @@ def load(build_if_missing: bool = True):
     L.mmw_default_radar_params.argtypes = [C.POINTER(RadarParams)]
     L.mmw_default_radar_params.restype = None
     L.mmw_to_physical.argtypes = [C.POINTER(RadarParams), C.c_int, C.c_int, vp, C.c_int, vp]
+    L.mmw_default_cluster_params.argtypes = [C.POINTER(ClusterParams)]
+    L.mmw_default_cluster_params.restype = None
+    L.mmw_set_clustering.argtypes = [vp, C.POINTER(ClusterParams)]
+    L.mmw_read_objects.argtypes = [vp, vp, C.c_int, ip]
+    L.mmw_read_labels.argtypes = [vp, vp, C.c_int, ip]
+    L.mmw_device_objects.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
+    L.mmw_objects_to_physical.argtypes = [C.POINTER(RadarParams), C.c_int, C.c_int, vp, C.c_int, vp]
     L.mmw_legacy_process_device.argtypes = [vp, C.c_int, vp, vp]
     L.mmw_legacy_distance_from_raw.argtypes = [C.c_int]
     L.mmw_legacy_distance_from_raw.restype = C.c_double
@@ -294,6 +324,47 @@ class RadarContext:
 
     def set_frame_offset(self, first_frame: int):
         _check(self._L.mmw_set_frame_offset(self._h, int(first_frame)))
+
+    def set_clustering(self, **params):
+        """Group each frame's detections into objects after every batch (include/mmw_radar.h: mmw_set_clustering).
+        Keyword arguments override mmw_default_cluster_params (eps_range, eps_doppler, eps_angle, min_points,
+        max_objects_per_frame); no arguments turn clustering off."""
+        if not params:
+            _check(self._L.mmw_set_clustering(self._h, None))
+        else:
+            cp = default_cluster_params()
+            for k, v in params.items():
+                if k not in dict(ClusterParams._fields_):
+                    raise TypeError(f"unknown clustering parameter {k!r}")
+                setattr(cp, k, int(v))
+            _check(self._L.mmw_set_clustering(self._h, C.byref(cp)))
+        _check(self._L.mmw_get_info(self._h, C.byref(self.info)))      # kernels_per_batch and workspace_bytes follow
+
+    def read_objects(self, capacity: int | None = None):
+        """Objects of the last (clustered) batch. Returns (objects, overflow_flag): overflow when objects were cut, the
+        detection list was truncated or capacity was short."""
+        cap = capacity if capacity is not None else self.max_frames * self.max_det_per_frame
+        objs = np.empty(max(cap, 1), OBJ_DTYPE)
+        n = C.c_int(0)
+        rc = _check(self._L.mmw_read_objects(self._h, _np_ptr(objs), cap, C.byref(n)), True)
+        return objs[: n.value].copy(), rc == MMW_ERR_OVERFLOW
+
+    def read_labels(self, capacity: int | None = None) -> np.ndarray:
+        """Object index of every detection of the last batch (aligned with its detection list), -1 for none."""
+        cap = capacity if capacity is not None else self.max_frames * self.max_det_per_frame
+        labels = np.empty(max(cap, 1), np.int32)
+        n = C.c_int(0)
+        _check(self._L.mmw_read_labels(self._h, _np_ptr(labels), cap, C.byref(n)))
+        return labels[: n.value].copy()
+
+    def device_objects(self):
+        """(device address of the object records, device address of the 32-byte object header)."""
+        o, h = C.c_void_p(), C.c_void_p()
+        _check(self._L.mmw_device_objects(self._h, C.byref(o), C.byref(h)))
+        return int(o.value), int(h.value)
+
+    def objects_to_physical(self, objs: np.ndarray, params: RadarParams | None = None) -> np.ndarray:
+        return objects_to_physical(objs, self.Sp, self.Cp, params)
 
     @property
     def stream(self) -> int:
@@ -577,6 +648,23 @@ def to_physical(dets: np.ndarray, Sp: int, Cp: int, params: RadarParams | None =
     d = np.ascontiguousarray(dets, DET_DTYPE)
     out = np.empty(d.size, TARGET_DTYPE)
     _check(L.mmw_to_physical(C.byref(params), Sp, Cp, _np_ptr(d), d.size, _np_ptr(out)))
+    return out
+
+
+def default_cluster_params() -> ClusterParams:
+    cp = ClusterParams()
+    load().mmw_default_cluster_params(C.byref(cp))
+    return cp
+
+
+def objects_to_physical(objs: np.ndarray, Sp: int, Cp: int, params: RadarParams | None = None) -> np.ndarray:
+    """Objects -> range [m], radial velocity [m/s], angle [deg] of their mean bins, SNR [dB] of their peak
+    (mmw_objects_to_physical; host arithmetic)."""
+    L = load()
+    params = params if params is not None else default_radar_params()
+    o = np.ascontiguousarray(objs, OBJ_DTYPE)
+    out = np.empty(o.size, TARGET_DTYPE)
+    _check(L.mmw_objects_to_physical(C.byref(params), Sp, Cp, _np_ptr(o), o.size, _np_ptr(out)))
     return out
 
 

@@ -13,7 +13,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libmmw_radar_b200.so")
-SOURCES = ["mmw_api.cu", "mmw_pipeline.cu", "mmw_detect.cu", "mmw_legacy.cu"]
+SOURCES = ["mmw_api.cu", "mmw_pipeline.cu", "mmw_detect.cu", "mmw_legacy.cu", "mmw_cluster.cu"]
 HEADERS = [
     os.path.join(CSRC, "fft_regs.cuh"),
     os.path.join(CSRC, "mmw_common.cuh"),

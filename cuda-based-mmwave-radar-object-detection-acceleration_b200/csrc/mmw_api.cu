@@ -110,6 +110,17 @@ struct mmw_ctx {
         uint32_t frame_offset;        // value `exec` currently holds
     };
     std::map<std::tuple<const void *, int, const void *, void *>, GraphEntry> *graphs;
+    // clustering (mmw_set_clustering): on when cluster_on; its buffers live from that call to the next one turning it off
+    int cluster_on;
+    mmw_cluster_params cluster;
+    int last_clustered;       // the last batch ran the clustering kernels
+    int *d_cl_parent, *d_cl_oid;
+    uint32_t *d_cl_size, *d_cl_cursor, *d_cl_members, *d_cl_frame_objs, *d_cl_obj_offsets;
+    int32_t *d_cl_labels;
+    uint2 *d_cl_slots;
+    unsigned int *d_cl_ticket;
+    unsigned char *d_objects;   // [MMW_OBJECT_HEADER_BYTES header | max_frames * max_objects_per_frame records]
+    size_t cluster_bytes;       // their share of workspace_bytes
 };
 
 static void destroy_graphs(mmw_ctx *c)
@@ -178,6 +189,21 @@ static void dev_free(mmw_ctx *c, void *user)
     cudaFree(user);
 }
 
+static void free_cluster_buffers(mmw_ctx *c)
+{
+    void *bufs[] = {c->d_cl_parent, c->d_cl_oid, c->d_cl_size, c->d_cl_cursor, c->d_cl_members, c->d_cl_frame_objs,
+                    c->d_cl_obj_offsets, c->d_cl_labels, c->d_cl_slots, c->d_cl_ticket, c->d_objects};
+    for (void *b : bufs) dev_free(c, b);
+    c->d_cl_parent = c->d_cl_oid = nullptr;
+    c->d_cl_size = c->d_cl_cursor = c->d_cl_members = c->d_cl_frame_objs = c->d_cl_obj_offsets = nullptr;
+    c->d_cl_labels = nullptr;
+    c->d_cl_slots = nullptr;
+    c->d_cl_ticket = nullptr;
+    c->d_objects = nullptr;
+    c->workspace_bytes -= c->cluster_bytes;
+    c->cluster_bytes = 0;
+}
+
 static std::vector<float2> make_twiddles(int n)
 {
     std::vector<float2> t(n);
@@ -240,6 +266,7 @@ void mmw_destroy(mmw_ctx *c)
                     c->d_psplit, c->d_mask, c->d_noise, c->d_keys, c->d_counts, c->d_offsets, c->d_ticket, c->d_sched,
                     c->d_rows, c->d_snap, c->d_result};
     for (void *b : bufs) dev_free(c, b);
+    free_cluster_buffers(c);
     cudaFree(c->d_scratch);
     delete c->guards;
     if (c->h_result) cudaFreeHost(c->h_result);
@@ -404,6 +431,7 @@ int mmw_get_info(const mmw_ctx *c, mmw_info *info)
     info->workspace_bytes = (long long)c->workspace_bytes;
     // K1, K2, K3, list, measure; the selective re-FFT path runs rows + extract + angle instead of measure
     info->kernels_per_batch = detect_uses_refft(p, c->d_rows != nullptr && c->d_snap != nullptr) ? 7 : 5;
+    if (c->cluster_on) info->kernels_per_batch += kClusterKernels;
     return MMW_OK;
 }
 
@@ -525,8 +553,19 @@ static int run_back(mmw_ctx *c, int n_frames, cudaEvent_t *stage_ev)
     b.keys = c->d_keys; b.counts = c->d_counts; b.offsets = c->d_offsets; b.header = c->d_header;
     b.ticket = c->d_ticket; b.dense = c->d_dense; b.rows = c->d_rows; b.snap = c->d_snap;
     CK(launch_detect(p, b, n_frames, c->dense_cap, c->sm_count, c->stream));
+    if (c->cluster_on) {
+        ClusterBuffers cb;
+        cb.dense = c->d_dense; cb.det_header = c->d_header; cb.keys = c->d_keys; cb.offsets = c->d_offsets;
+        cb.parent = c->d_cl_parent; cb.size = c->d_cl_size; cb.oid = c->d_cl_oid; cb.cursor = c->d_cl_cursor;
+        cb.members = c->d_cl_members; cb.labels = c->d_cl_labels; cb.frame_objs = c->d_cl_frame_objs;
+        cb.obj_offsets = c->d_cl_obj_offsets; cb.slots = c->d_cl_slots; cb.ticket = c->d_cl_ticket;
+        cb.obj_header = reinterpret_cast<uint32_t *>(c->d_objects);
+        cb.objs = reinterpret_cast<mmw_object *>(c->d_objects + MMW_OBJECT_HEADER_BYTES);
+        CK(launch_cluster(c->cluster, p.Cp, p.max_det, cb, n_frames, c->dense_cap, c->sm_count, c->stream));
+    }
     if (stage_ev) CK(cudaEventRecord(stage_ev[4], c->stream));
     c->last_frames = n_frames;
+    c->last_clustered = c->cluster_on;
     return MMW_OK;
 }
 
@@ -600,6 +639,7 @@ static int run_batch_graphed(mmw_ctx *c, const int16_t *adc_dev, int n_frames)
     }
     CK(cudaGraphLaunch(ge.exec, c->stream));
     c->last_frames = n_frames;
+    c->last_clustered = c->cluster_on;
     return MMW_OK;
 }
 
@@ -838,27 +878,188 @@ void mmw_default_radar_params(mmw_radar_params *rp)
     rp->light_speed = 3.0e8;
 }
 
-int mmw_to_physical(const mmw_radar_params *rp, int Sp, int Cp, const mmw_detection *dets, int n, mmw_target *out)
+// the bin -> metre and bin -> m/s formulas of mmw_to_physical and mmw_objects_to_physical (a fractional bin takes the same
+// expression; an integer bin converts to double exactly)
+static float range_bin_to_m(const mmw_radar_params *rp, int Sp, double range_bin)
 {
-    if (!rp || Sp < 1 || Cp < 1 || n < 0 || (n > 0 && (!dets || !out))) { set_last_error("mmw_to_physical: bad argument"); return MMW_ERR_ARG; }
+    const double f_beat = range_bin / (double)Sp * rp->fs_hz;
+    return (float)(rp->light_speed * f_beat / (2.0 * rp->slope_hz_per_s));
+}
+
+static float doppler_bin_to_mps(const mmw_radar_params *rp, int Cp, double signed_doppler_bin)
+{
+    const double lambda = rp->light_speed / rp->f0_hz;
+    const double f_dop = signed_doppler_bin / ((double)Cp * rp->chirp_period_s);
+    return (float)(0.5 * lambda * f_dop);
+}
+
+static int check_radar_params(const mmw_radar_params *rp, int Sp, int Cp, int n, const void *in, const void *out, const char *who)
+{
+    if (!rp || Sp < 1 || Cp < 1 || n < 0 || (n > 0 && (!in || !out))) { set_last_error("%s: bad argument", who); return MMW_ERR_ARG; }
     if (rp->f0_hz <= 0 || rp->slope_hz_per_s <= 0 || rp->fs_hz <= 0 || rp->chirp_period_s <= 0 || rp->light_speed <= 0) {
-        set_last_error("mmw_to_physical: radar parameters must be positive");
+        set_last_error("%s: radar parameters must be positive", who);
         return MMW_ERR_ARG;
     }
-    const double lambda = rp->light_speed / rp->f0_hz;
+    return MMW_OK;
+}
+
+int mmw_to_physical(const mmw_radar_params *rp, int Sp, int Cp, const mmw_detection *dets, int n, mmw_target *out)
+{
+    const int rc = check_radar_params(rp, Sp, Cp, n, dets, out, "mmw_to_physical");
+    if (rc) return rc;
     for (int i = 0; i < n; ++i) {
         const mmw_detection &d = dets[i];
-        const double f_beat = (double)d.range_bin / (double)Sp * rp->fs_hz;
         const int dw = d.doppler_bin < Cp / 2 ? (int)d.doppler_bin : (int)d.doppler_bin - Cp;
-        const double f_dop = (double)dw / ((double)Cp * rp->chirp_period_s);
         mmw_target &t = out[i];
         t.frame = d.frame;
-        t.range_m = (float)(rp->light_speed * f_beat / (2.0 * rp->slope_hz_per_s));
-        t.velocity_mps = (float)(0.5 * lambda * f_dop);
+        t.range_m = range_bin_to_m(rp, Sp, (double)d.range_bin);
+        t.velocity_mps = doppler_bin_to_mps(rp, Cp, (double)dw);
         t.angle_deg = (float)((double)d.angle_rad * (180.0 / M_PI));
         t.snr_db = (d.noise > 0.f && d.power > 0.f) ? (float)(10.0 * log10((double)d.power / (double)d.noise)) : 0.f;
         t.flags = d.flags;
     }
+    return MMW_OK;
+}
+
+int mmw_objects_to_physical(const mmw_radar_params *rp, int Sp, int Cp, const mmw_object *objs, int n, mmw_target *out)
+{
+    const int rc = check_radar_params(rp, Sp, Cp, n, objs, out, "mmw_objects_to_physical");
+    if (rc) return rc;
+    for (int i = 0; i < n; ++i) {
+        const mmw_object &o = objs[i];
+        mmw_target &t = out[i];
+        t.frame = o.frame;
+        t.range_m = range_bin_to_m(rp, Sp, (double)o.range_bin);
+        t.velocity_mps = doppler_bin_to_mps(rp, Cp, (double)o.doppler_bin);
+        t.angle_deg = (float)((double)o.angle_rad * (180.0 / M_PI));
+        t.snr_db = (o.peak_noise > 0.f && o.peak_power > 0.f) ? (float)(10.0 * log10((double)o.peak_power / (double)o.peak_noise)) : 0.f;
+        t.flags = 0;
+    }
+    return MMW_OK;
+}
+
+// ---------------------------------------------------------------------------
+// clustering of each frame's detections into objects (kernels: mmw_cluster.cu)
+// ---------------------------------------------------------------------------
+void mmw_default_cluster_params(mmw_cluster_params *cp)
+{
+    if (!cp) return;
+    cp->eps_range = 2;
+    cp->eps_doppler = 2;
+    cp->eps_angle = 4;
+    cp->min_points = 1;
+    cp->max_objects_per_frame = 256;
+}
+
+int mmw_set_clustering(mmw_ctx *c, const mmw_cluster_params *cp)
+{
+    if (!c) { set_last_error("mmw_set_clustering: null context"); return MMW_ERR_ARG; }
+    if (cp) {
+        if (cp->eps_range < 0 || cp->eps_range > 16) { set_last_error("mmw_set_clustering: eps_range must be 0..16, got %d", cp->eps_range); return MMW_ERR_ARG; }
+        if (cp->eps_doppler < 0 || cp->eps_doppler > 16) { set_last_error("mmw_set_clustering: eps_doppler must be 0..16, got %d", cp->eps_doppler); return MMW_ERR_ARG; }
+        if (cp->eps_angle < 0) { set_last_error("mmw_set_clustering: eps_angle must be >= 0, got %d", cp->eps_angle); return MMW_ERR_ARG; }
+        if (cp->min_points < 1) { set_last_error("mmw_set_clustering: min_points must be >= 1, got %d", cp->min_points); return MMW_ERR_ARG; }
+        if (cp->max_objects_per_frame < 1 || cp->max_objects_per_frame > c->cfg.max_det_per_frame) {
+            set_last_error("mmw_set_clustering: max_objects_per_frame must be 1..max_det_per_frame (%d), got %d", c->cfg.max_det_per_frame,
+                           cp->max_objects_per_frame);
+            return MMW_ERR_ARG;
+        }
+    }
+    if (c->submitted) { set_last_error("mmw_set_clustering: a submitted batch is pending; collect it with mmw_wait"); return MMW_ERR_STATE; }
+    CK(cudaSetDevice(c->device));
+    CK(cudaStreamSynchronize(c->stream));               // a batch in flight may still use the buffers
+    if (c->graphs) destroy_graphs(c);                  // the captured launch sequences belong to the old setting
+    const bool same_capacity = cp && c->cluster_on && c->cluster.max_objects_per_frame == cp->max_objects_per_frame;
+    if (!same_capacity) {
+        free_cluster_buffers(c);
+        c->cluster_on = 0;
+        c->last_clustered = 0;
+    }
+    if (!cp) return MMW_OK;
+    if (!same_capacity) {
+        const size_t D = (size_t)c->dense_cap, F = (size_t)c->cfg.max_frames;
+        const size_t obj_cap = F * (size_t)cp->max_objects_per_frame;
+        const size_t before = c->workspace_bytes;
+        int rc;
+        if ((rc = dev_alloc(c, &c->d_cl_parent, D)) || (rc = dev_alloc(c, &c->d_cl_size, D)) || (rc = dev_alloc(c, &c->d_cl_oid, D)) ||
+            (rc = dev_alloc(c, &c->d_cl_cursor, D)) || (rc = dev_alloc(c, &c->d_cl_members, D)) || (rc = dev_alloc(c, &c->d_cl_labels, D)) ||
+            (rc = dev_alloc(c, &c->d_cl_frame_objs, 2 * F)) || (rc = dev_alloc(c, &c->d_cl_obj_offsets, F + 1)) ||
+            (rc = dev_alloc(c, &c->d_cl_slots, obj_cap)) || (rc = dev_alloc(c, &c->d_cl_ticket, (size_t)1)) ||
+            (rc = dev_alloc(c, &c->d_objects, (size_t)MMW_OBJECT_HEADER_BYTES + obj_cap * sizeof(mmw_object)))) {
+            c->cluster_bytes = c->workspace_bytes - before;
+            free_cluster_buffers(c);
+            return rc;
+        }
+        c->cluster_bytes = c->workspace_bytes - before;
+        // the ticket self-resets after every batch; the header reads "no objects" until the first clustered batch
+        CK(cudaMemset(c->d_cl_ticket, 0, sizeof(unsigned int)));
+        CK(cudaMemset(c->d_objects, 0, MMW_OBJECT_HEADER_BYTES));
+    }
+    c->cluster = *cp;
+    c->cluster_on = 1;
+    return MMW_OK;
+}
+
+static int check_clustered(mmw_ctx *c, const char *who)
+{
+    if (!c) { set_last_error("%s: null context", who); return MMW_ERR_ARG; }
+    if (c->submitted) { set_last_error("%s: a submitted batch is pending; collect it with mmw_wait", who); return MMW_ERR_STATE; }
+    if (!c->cluster_on || !c->last_clustered || c->last_frames <= 0) {
+        set_last_error("%s: the last batch was not clustered (mmw_set_clustering)", who);
+        return MMW_ERR_STATE;
+    }
+    return MMW_OK;
+}
+
+int mmw_read_objects(mmw_ctx *c, mmw_object *objs, int capacity, int *n_obj)
+{
+    int rc = check_clustered(c, "mmw_read_objects");
+    if (rc) return rc;
+    if (capacity < 0 || (capacity > 0 && !objs)) { set_last_error("mmw_read_objects: bad capacity / null output"); return MMW_ERR_ARG; }
+    CK(cudaSetDevice(c->device));
+    uint32_t hdr[MMW_OBJECT_HEADER_BYTES / 4];
+    CK(cudaMemcpyAsync(hdr, c->d_objects, sizeof(hdr), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    uint32_t n = hdr[0];
+    rc = hdr[3] ? MMW_ERR_OVERFLOW : MMW_OK;
+    if ((long long)n > (long long)capacity) { n = (uint32_t)capacity; rc = MMW_ERR_OVERFLOW; }
+    if (n > 0) {
+        CK(cudaMemcpyAsync(objs, c->d_objects + MMW_OBJECT_HEADER_BYTES, (size_t)n * sizeof(mmw_object), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+    }
+    if (n_obj) *n_obj = (int)n;
+    if (rc == MMW_ERR_OVERFLOW)
+        set_last_error("object list incomplete: %u of %u objects kept (flags 0x%x)", n, hdr[1], hdr[3]);
+    return rc;
+}
+
+int mmw_read_labels(mmw_ctx *c, int32_t *labels, int capacity, int *n)
+{
+    int rc = check_clustered(c, "mmw_read_labels");
+    if (rc) return rc;
+    if (capacity < 0 || (capacity > 0 && !labels)) { set_last_error("mmw_read_labels: bad capacity / null output"); return MMW_ERR_ARG; }
+    CK(cudaSetDevice(c->device));
+    uint32_t n_written = 0;
+    CK(cudaMemcpyAsync(&n_written, c->d_header, sizeof(n_written), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    uint32_t k = n_written;
+    rc = MMW_OK;
+    if ((long long)k > (long long)capacity) { k = (uint32_t)capacity; rc = MMW_ERR_OVERFLOW; }
+    if (k > 0) {
+        CK(cudaMemcpyAsync(labels, c->d_cl_labels, (size_t)k * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+    }
+    if (n) *n = (int)k;
+    if (rc == MMW_ERR_OVERFLOW) set_last_error("mmw_read_labels: %u labels, capacity %d", n_written, capacity);
+    return rc;
+}
+
+int mmw_device_objects(mmw_ctx *c, const mmw_object **objs, const uint32_t **header)
+{
+    if (!c) { set_last_error("mmw_device_objects: null context"); return MMW_ERR_ARG; }
+    if (!c->cluster_on) { set_last_error("mmw_device_objects: clustering is off (mmw_set_clustering)"); return MMW_ERR_STATE; }
+    if (objs) *objs = reinterpret_cast<const mmw_object *>(c->d_objects + MMW_OBJECT_HEADER_BYTES);
+    if (header) *header = reinterpret_cast<const uint32_t *>(c->d_objects);
     return MMW_OK;
 }
 

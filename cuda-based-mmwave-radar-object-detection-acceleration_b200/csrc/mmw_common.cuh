@@ -133,6 +133,28 @@ cudaError_t launch_doppler_extract(const PlanDev &p, const float2 *rs, const uin
                                    const unsigned int *n_rows, float2 *snap, int dense_cap, int max_rows, cudaStream_t st);
 cudaError_t launch_merge(const unsigned char *gathered, int n_ranks, size_t stride_bytes, unsigned char *merged, int merged_cap,
                          cudaStream_t st);
+// clustering of the finished detection list into objects (mmw_cluster.cu); every buffer is [dense capacity] unless noted
+struct ClusterBuffers {
+    const mmw_detection *dense;     // the batch's detection list, its header {n_written, n_total, n_frames, overflow}
+    const uint32_t *det_header;
+    const uint32_t *keys;           // [F][max_det] (range << 16 | doppler) of list_kernel, offsets [F+1]
+    const uint32_t *offsets;
+    int *parent;                    // union-find forest; after the flatten pass the component root (its lowest index)
+    uint32_t *size;                 // component size, at the root
+    int *oid;                       // at a root: frame-local object number, -1 if the component is not an object
+    uint32_t *cursor;               // at a kept root: next free slot of its members in `members`
+    uint32_t *members;              // member indices grouped by object, ascending within each object
+    int32_t *labels;                // object index per detection, -1 if none
+    uint32_t *frame_objs;           // [2F] objects per frame: true count, kept count
+    uint32_t *obj_offsets;          // [F+1] exclusive scan of the kept counts
+    uint2 *slots;                   // [F][max_obj] {root, first member slot} of each kept object
+    unsigned int *ticket;           // [1] last-CTA-done counter of the order kernel (self-resetting)
+    uint32_t *obj_header;           // MMW_OBJECT_HEADER_BYTES
+    mmw_object *objs;               // [F][max_obj] capacity
+};
+constexpr int kClusterKernels = 5;
+cudaError_t launch_cluster(const mmw_cluster_params &cp, int Cp, int max_det, const ClusterBuffers &b, int n_frames, int dense_cap,
+                           int sm_count, cudaStream_t st);
 // export helpers (not on the hot path): internal layout -> the canonical layouts of mmw_radar.h
 cudaError_t launch_export_cube(const PlanDev &p, const float2 *cube_frame, float2 *out, cudaStream_t st);
 cudaError_t launch_export_pmap(const PlanDev &p, const float *pmap_frame, float *out, cudaStream_t st);

@@ -250,6 +250,69 @@ void mmw_default_radar_params(mmw_radar_params *rp);
 /* Sp, Cp: the FFT lengths the detections were made with (mmw_info.Sp / .Cp) */
 int mmw_to_physical(const mmw_radar_params *rp, int Sp, int Cp, const mmw_detection *dets, int n, mmw_target *out);
 
+/* ---- clustering: each frame's detections grouped into objects, on the GPU (off by default) ----
+ * One target under the Hann windows lights up a blob of neighbouring cells; MMW_FLAG_PEAK marks the blob's maximum but not
+ * its members.  With clustering on, every batch also produces an ordered object list and a label per detection.
+ * Definition (tests/cluster_ref.c: ref_cluster, a plain-C fp64 reference, is the specification; the GPU matches it bit for bit):
+ *   signed Doppler d' = d < Cp/2 ? d : d - Cp, without wrap: a blob that straddles +-Cp/2 becomes two objects;
+ *   detections i, j of one frame are neighbours iff |r_i - r_j| <= eps_range, |d'_i - d'_j| <= eps_doppler and
+ *   |angle_bin_i - angle_bin_j| <= eps_angle (eps_angle >= n_theta ignores the angle);
+ *   components of the neighbour graph (friends-of-friends: DBSCAN with min_points = 1, unique whatever the order) with at
+ *   least min_points members are objects, ordered by (frame, lowest member index); at most max_objects_per_frame per frame
+ *   are kept, the true count is always reported.
+ * The kernels read the finished detection list and write their own buffers only: the detections are the same bytes with
+ * clustering on or off.  They run at the end of every batch (mmw_process_device / _host, mmw_submit_host, capture-file
+ * ingest, graph mode) and mmw_time_device counts them in stage 4.
+ * Multi-GPU: mmw_group_* and mmw_exchange_* gather detections only; enable clustering on each mmw_group_context() and read
+ * the objects of each shard from that context. */
+typedef struct mmw_cluster_params {
+    int eps_range;              /* 0..16 range bins */
+    int eps_doppler;            /* 0..16 Doppler bins (signed, no wrap) */
+    int eps_angle;              /* >= 0 angle bins; >= n_theta: angle ignored */
+    int min_points;             /* >= 1 detections per object */
+    int max_objects_per_frame;  /* 1..max_det_per_frame */
+} mmw_cluster_params;
+
+/* 48-byte object record.  Sums run over the members in ascending detection index, in fp64, rounded to fp32 once. */
+typedef struct mmw_object {
+    uint32_t frame;        /* the members' mmw_detection.frame (frame offset included) */
+    uint32_t first_det;    /* index of the lowest-index member in the batch's detection list */
+    uint32_t n_det;        /* members */
+    uint32_t peak_det;     /* index of the strongest member (equal power: the lower index) */
+    float range_bin;       /* power-weighted mean range bin */
+    float doppler_bin;     /* power-weighted mean signed Doppler bin d' */
+    float angle_rad;       /* power-weighted mean angle_rad */
+    float power;           /* sum of the members' power */
+    float peak_power;      /* power and noise of peak_det */
+    float peak_noise;
+    uint16_t range_min, range_max;
+    int16_t doppler_min, doppler_max;   /* signed d' */
+} mmw_object;
+
+/* object header: {n_written, n_total, n_frames, flags} + 4 reserved words; flags bit 0: some frame had more than
+ * max_objects_per_frame objects (those were cut), bit 1: the detection list itself was truncated (max_det_per_frame) */
+#define MMW_OBJECT_HEADER_BYTES 32
+#define MMW_OBJECTS_CUT 0x1u
+#define MMW_OBJECTS_DETECTIONS_TRUNCATED 0x2u
+
+/* (2, 2, 4, 1, 256) */
+void mmw_default_cluster_params(mmw_cluster_params *cp);
+/* cp = NULL turns clustering off (the default) and releases its buffers; otherwise checks the parameters, allocates the
+ * buffers (all of them: nothing is allocated inside a batch, which may be under stream capture) and turns it on.
+ * MMW_ERR_STATE while a submitted batch is pending.  Call between batches. */
+int mmw_set_clustering(mmw_ctx *ctx, const mmw_cluster_params *cp);
+/* After a batch with clustering on: synchronises, copies up to `capacity` objects.  Returns MMW_ERR_OVERFLOW (after
+ * filling objs) if the header has a flag set or there were more than `capacity` objects. */
+int mmw_read_objects(mmw_ctx *ctx, mmw_object *objs, int capacity, int *n_obj);
+/* Per detection of the last batch (aligned with its detection list): the index of its object in the object list, or -1
+ * (its component is smaller than min_points, or its object was cut).  MMW_ERR_OVERFLOW if capacity < detections. */
+int mmw_read_labels(mmw_ctx *ctx, int32_t *labels, int capacity, int *n);
+/* device views: *objs at the object records, *header at the MMW_OBJECT_HEADER_BYTES header right before them */
+int mmw_device_objects(mmw_ctx *ctx, const mmw_object **objs, const uint32_t **header);
+/* objects in physical units with mmw_to_physical's formulas applied to the fractional mean bins; snr_db is
+ * 10 log10(peak_power / peak_noise), flags is 0 */
+int mmw_objects_to_physical(const mmw_radar_params *rp, int Sp, int Cp, const mmw_object *objs, int n, mmw_target *out);
+
 /* Intermediates of one frame of the last batch, copied to the host in canonical layouts
  * (synchronous, not on the hot path):
  *   range spectrum [A][Sp][C]  complex64 — NOTE: already multiplied by the Doppler window w_d[c]
@@ -264,7 +327,8 @@ int mmw_copy_cfar_mask(mmw_ctx *ctx, int frame, uint8_t *out);
 /* Device timing helper: runs mmw_process_device `iters` times back to back on the context
  * stream between two CUDA events and returns the elapsed milliseconds (total, not per run).
  * per_stage_ms (optional, 4 floats) receives the summed time of each stage
- * (range, doppler, cfar, detect+compact) measured with events between the launches. */
+ * (range, doppler, cfar, detect+compact, plus the clustering kernels when clustering is on) measured with events between
+ * the launches. */
 int mmw_time_device(mmw_ctx *ctx, const int16_t *adc_dev, int n_frames, int iters,
                     float *total_ms, float *per_stage_ms);
 
