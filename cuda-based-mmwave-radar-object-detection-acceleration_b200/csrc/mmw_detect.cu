@@ -332,7 +332,10 @@ static cudaError_t run_cfar_walk(const PlanDev &p, const float *pmap, uint32_t *
     case 256:  return run_cfar_walk_t<RT, MINB, 256>(p, pmap, mask, noise_map, nchunk, n_frames, st);
     case 512:  return run_cfar_walk_t<RT, MINB, 512>(p, pmap, mask, noise_map, nchunk, n_frames, st);
     case 1024: return run_cfar_walk_t<RT, MINB, 1024>(p, pmap, mask, noise_map, nchunk, n_frames, st);
-    default:   return run_cfar_walk_t<RT, MINB, 0>(p, pmap, mask, noise_map, nchunk, n_frames, st);
+    default:
+        // 256-bin strips need Sp % 256 == 0, and every such Sp has its own specialisation above: no run-time-Sp form
+        if constexpr (RT == 256) return cudaErrorInvalidValue;
+        else return run_cfar_walk_t<RT, MINB, 0>(p, pmap, mask, noise_map, nchunk, n_frames, st);
     }
 }
 

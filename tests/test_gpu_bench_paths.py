@@ -14,32 +14,14 @@ Here the batch sizes are the bench's, so the kernels checked are the kernels tim
   cfg4  1024 x 512 x 192, 1 frame   range<1024,..,CT=512>, doppler<512,..,SPT=1024, in place, 3 stages>,
                                     measure_wide_kernel / the selective Doppler re-FFT, 256-point angle FFT
 
-Tolerances (north_star: fp32 relative error 1e-4 for FFT outputs and power maps; CFAR indices bit-exact except cells
-within 1e-5 relative of threshold, which are listed):
-  power map   |P - P_ref| <= 2e-6 * max(P_ref) everywhere, AND per-bin relative error <= 1e-5 for every bin above
-              1e-3 * max(P_ref) (per-bin relative error is meaningless on near-empty bins: SURVEY.md §7); the measured
-              maxima are printed (north_star's bound is 1e-4)
-  CFAR mask   bit-exact except cells with |P - alpha * noise| <= 1e-5 * alpha * noise (counted and printed)
-  list        keys (frame, range, doppler) in order, identical to the oracle's away from those cells; counts exact
-  noise       relative error <= NOISE_RTOL (see below) at every detection
-  angle bin   identical unless the oracle's angle spectrum has a second bin within 1e-4 of the maximum
-  peak flag   identical unless a detected neighbour's power is within 1e-4 of the cell's, or a threshold cell is adjacent
+Tolerances: tests/chain_check.py, which holds the comparison (check_frames) this file and test_gpu_kernel_forms.py share.
 """
 import numpy as np
 import pytest
 
-pytestmark = pytest.mark.gpu
+from chain_check import check_frames
 
-ALPHA = 15.0
-NEAR = 1e-5
-P_ATOL_OF_MAX = 2e-6            # measured on B200: 1.6e-7 .. 3.7e-7 (profiles/r2/parity_maxima_bench_paths.log: this file run with -s)
-P_RTOL_ABOVE_FLOOR = 1e-5       # measured: 2.4e-7 .. 7.0e-7; north_star allows 1e-4
-P_FLOOR_OF_MAX = 1e-3
-# The noise estimate is the mean of 248 power-map cells near the noise floor.  Its fp32 sum is add-only (~1e-6), but
-# each of those cells carries the fp32 FFT's error, which is relative to the RMS of the whole transform (dominated by
-# targets ~1e9 x the floor), not to the cell: ~1e-4 per cell, averaging down over the window.  Measured on B200: 1.4e-6 ..
-# 1.05e-5 (the largest on one of the 7 858 detections of the cfg3 batch).
-NOISE_RTOL = 3e-5
+pytestmark = pytest.mark.gpu
 
 
 def _torch_batch(pkg, F, S, C, A, cfg, first_frame=0, n_targets=8):
@@ -52,73 +34,6 @@ def _torch_batch(pkg, F, S, C, A, cfg, first_frame=0, n_targets=8):
     return out
 
 
-def _check_frames(pkg, orc, ctx, dets, adc, frames, S, C, A, tag, n_threads=8):
-    """compares frames `frames` of the batch just processed on `ctx` (detections `dets`) with the oracle run on those frames"""
-    wr, wd = ctx.get_windows()
-    sub = np.ascontiguousarray(adc[frames])
-    ref = orc.process_frames(sub, len(frames), S, C, A, wr, wd, want=("P", "mask", "noise", "ratio"), n_threads=n_threads,
-                             det_cap_per_frame=ctx.max_det_per_frame)
-    stats = dict(p_abs=0.0, p_rel=0.0, near=0, n_det=0, noise_rel=0.0, angle_ties=0, flag_skipped=0)
-    for i, f in enumerate(frames):
-        Pr, maskr, noiser = ref["P"][i], ref["mask"][i], ref["noise"][i]
-        P = ctx.power_map(f).astype(np.float64)
-        pmax = Pr.max()
-        err = np.abs(P - Pr)
-        stats["p_abs"] = max(stats["p_abs"], float(err.max() / pmax))
-        assert err.max() <= P_ATOL_OF_MAX * pmax, f"{tag} frame {f}: power map off by {err.max() / pmax:.2e} of its maximum"
-        big = Pr >= P_FLOOR_OF_MAX * pmax
-        rel = float((err[big] / Pr[big]).max())
-        stats["p_rel"] = max(stats["p_rel"], rel)
-        assert rel <= P_RTOL_ABOVE_FLOOR, f"{tag} frame {f}: per-bin relative error {rel:.2e} above the floor"
-        thr = ALPHA * noiser
-        near = np.abs(Pr - thr) <= NEAR * thr
-        stats["near"] += int(near.sum())
-        m = ctx.cfar_mask(f)
-        bad = (m != maskr) & ~near
-        assert not bad.any(), f"{tag} frame {f}: {int(bad.sum())} CFAR cells differ away from threshold"
-        # detection list of this frame
-        got = dets[dets["frame"] == f]
-        want = ref["dets"][ref["dets"]["frame"] == i]
-        ratio = ref["ratio"][ref["dets"]["frame"] == i]
-        assert len(got) == int(m.sum()), f"{tag} frame {f}: list length {len(got)} != mask population {int(m.sum())}"
-        gk = got["range_bin"].astype(np.int64) << 16 | got["doppler_bin"]
-        wk = want["range_bin"].astype(np.int64) << 16 | want["doppler_bin"]
-        assert np.all(np.diff(gk) > 0), f"{tag} frame {f}: list not ordered by (range, doppler)"
-        diff = np.setxor1d(gk, wk)
-        assert all(near[k >> 16, k & 0xffff] for k in diff), f"{tag} frame {f}: hit list differs away from threshold cells"
-        common, gi, wi = np.intersect1d(gk, wk, return_indices=True)
-        g, w, rt = got[gi], want[wi], ratio[wi]
-        stats["n_det"] += len(common)
-        assert len(common) > 0, f"{tag} frame {f}: no detections to compare"
-        assert np.abs(g["power"].astype(np.float64) - w["power"]).max() <= P_ATOL_OF_MAX * pmax
-        nrel = np.abs(g["noise"].astype(np.float64) - w["noise"]) / w["noise"]
-        stats["noise_rel"] = max(stats["noise_rel"], float(nrel.max()))
-        assert nrel.max() <= NOISE_RTOL, f"{tag} frame {f}: noise estimate off by {nrel.max():.2e} (relative)"
-        clear = rt < 1 - 1e-4
-        stats["angle_ties"] += int((~clear).sum())
-        assert np.array_equal(g["angle_bin"][clear], w["angle_bin"][clear]), f"{tag} frame {f}: angle bins differ away from ties"
-        assert np.abs(g["angle_rad"][clear] - w["angle_rad"][clear]).max(initial=0.0) < 1e-5
-        # grouping flag
-        Sp, Cp = Pr.shape
-        r, d = w["range_bin"].astype(np.int64), w["doppler_bin"].astype(np.int64)
-        ok = np.ones(len(w), bool)
-        for dr in (-1, 0, 1):
-            for dd in (-1, 0, 1):
-                rr, dn = r + dr, (d + dd) % Cp
-                inside = (rr >= 0) & (rr < Sp)
-                rr = rr.clip(0, Sp - 1)
-                ok &= ~(inside & near[rr, dn])
-                if dr or dd:
-                    close = inside & (maskr[rr, dn] != 0) & (np.abs(Pr[rr, dn] - Pr[r, d]) <= 1e-4 * Pr[r, d])
-                    ok &= ~close
-        stats["flag_skipped"] += int((~ok).sum())
-        assert np.array_equal(g["flags"][ok] & 1, w["flags"][ok] & 1), f"{tag} frame {f}: peak flags differ"
-    print(f"\n{tag}: frames {list(frames)}: {stats['n_det']} detections compared; power map max error {stats['p_abs']:.2e} of max, "
-          f"{stats['p_rel']:.2e} per bin above {P_FLOOR_OF_MAX} of max; noise max rel error {stats['noise_rel']:.2e}; "
-          f"{stats['near']} threshold cells excluded, {stats['angle_ties']} angle ties, {stats['flag_skipped']} flags skipped")
-    return stats
-
-
 def test_cfg3_bench_batch_fused(pkg, orc):
     """cfg3 at the bench's 64 frames per batch, fused mode: every frame's power map, mask and list against the oracle"""
     S, C, A, F = 512, 256, 12, 64
@@ -126,7 +41,7 @@ def test_cfg3_bench_batch_fused(pkg, orc):
     with pkg.RadarContext(S, C, A, F, max_det_per_frame=4096) as ctx:
         dets, overflow = ctx.process_host(adc, F)
         assert not overflow
-        _check_frames(pkg, orc, ctx, dets, adc, list(range(F)), S, C, A, "cfg3 x64 fused", n_threads=16)
+        check_frames(pkg, orc, ctx, dets, adc, list(range(F)), S, C, A, "cfg3 x64 fused", n_threads=16)
         # the device-resident entry point the bench times gives the same bytes
         import torch
 
@@ -143,7 +58,7 @@ def test_cfg3_bench_batch_with_cube(pkg, orc):
     with pkg.RadarContext(S, C, A, F, max_det_per_frame=4096, keep_doppler_cube=True) as ctx:
         dets, overflow = ctx.process_host(adc, F)
         assert not overflow
-        _check_frames(pkg, orc, ctx, dets, adc, [0, 7, 15], S, C, A, "cfg3 x16 cube", n_threads=8)
+        check_frames(pkg, orc, ctx, dets, adc, [0, 7, 15], S, C, A, "cfg3 x16 cube", n_threads=8)
 
 
 def test_cfg2_bench_batch_sampled_frames(pkg, orc):
@@ -159,7 +74,7 @@ def test_cfg2_bench_batch_sampled_frames(pkg, orc):
             assert int(ctx.info.kernels_per_batch) == (7 if path == pkg.api.DETECT_REFFT else 5)
             dets, overflow = ctx.process_host(adc, F)
             assert not overflow
-            _check_frames(pkg, orc, ctx, dets, adc, [517, 1023], S, C, A, f"cfg2 x1024 {tag}")
+            check_frames(pkg, orc, ctx, dets, adc, [517, 1023], S, C, A, f"cfg2 x1024 {tag}")
             lists[path] = dets.copy()
     a, b = lists[pkg.api.DETECT_REFFT], lists[pkg.api.DETECT_PER_CELL]
     assert len(a) == len(b)
@@ -178,7 +93,7 @@ def test_cfg5_sensor_cube_batch_and_single_calls(pkg, orc):
     with pkg.RadarContext(S, C, A, F, max_det_per_frame=4096) as ctx:
         dets, overflow = ctx.process_host(adc, F)
         assert not overflow
-        _check_frames(pkg, orc, ctx, dets, adc, list(range(F)), S, C, A, "cfg5 x8")
+        check_frames(pkg, orc, ctx, dets, adc, list(range(F)), S, C, A, "cfg5 x8")
     for graph in (False, True):
         with pkg.RadarContext(S, C, A, 1, max_det_per_frame=4096) as ctx:
             ctx.set_graph_mode(graph)
@@ -190,7 +105,7 @@ def test_cfg5_sensor_cube_batch_and_single_calls(pkg, orc):
             assert one.tobytes() == dets.tobytes(), f"one frame per call (graph={graph}) differs from the batch"
             ctx.set_frame_offset(0)
             d0, _ = ctx.process_host(adc[3], 1)
-            _check_frames(pkg, orc, ctx, d0, adc[3:4], [0], S, C, A, f"cfg5 single call graph={graph}")
+            check_frames(pkg, orc, ctx, d0, adc[3:4], [0], S, C, A, f"cfg5 single call graph={graph}")
 
 
 def test_cfg4_full_imaging_frame(pkg, orc):
@@ -202,4 +117,4 @@ def test_cfg4_full_imaging_frame(pkg, orc):
         assert not overflow
         counts = ctx.read_counts(F)
         assert counts[0] == len(dets) > 0
-        _check_frames(pkg, orc, ctx, dets, adc, [0], S, C, A, "cfg4 x1", n_threads=1)
+        check_frames(pkg, orc, ctx, dets, adc, [0], S, C, A, "cfg4 x1", n_threads=1)

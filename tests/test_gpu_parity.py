@@ -5,6 +5,8 @@ of their threshold, which are counted and printed; integer/index work bit-exact.
 import numpy as np
 import pytest
 
+from chain_check import WALK_FORMS, cfar_form_name, launched_kernels
+
 pytestmark = pytest.mark.gpu
 
 TOL = 1e-4          # relative to the maximum of the array being compared
@@ -118,10 +120,15 @@ def test_cfar_and_detections(pkg, orc, cases, shape, keep):
             assert (d["flags"] & 1) == (o["flags"] & 1)
 
 
-@pytest.mark.parametrize("guard,train,alpha", [((0, 0), (1, 1), 6.0), ((1, 3), (5, 2), 10.0), ((4, 1), (12, 7), 12.0), ((2, 2), (8, 4), 4.0)])
-def test_cfar_geometries(pkg, orc, guard, train, alpha):
+# the last two: the largest windows mmw_create accepts (guard + train = 64 range bins; 31 Doppler bins at Cp = 64, 32 at
+# Cp >= 128): the halo covers most of the map, and every row's range window is clamped where the Doppler window wraps
+@pytest.mark.parametrize("shape,guard,train,alpha", [((128, 64, 4, 2), (0, 0), (1, 1), 6.0), ((128, 64, 4, 2), (1, 3), (5, 2), 10.0),
+                                                     ((128, 64, 4, 2), (4, 1), (12, 7), 12.0), ((128, 64, 4, 2), (2, 2), (8, 4), 4.0),
+                                                     ((128, 64, 4, 2), (4, 3), (60, 28), 4.0), ((256, 128, 2, 2), (1, 2), (63, 30), 4.0)],
+                         ids=lambda v: "x".join(map(str, v)) if isinstance(v, tuple) else str(v))
+def test_cfar_geometries(pkg, orc, shape, guard, train, alpha):
     """non-default guard / training windows take the run-time-bound CFAR path; range edges clamp, Doppler wraps"""
-    S, C, A, F = 128, 64, 4, 2
+    S, C, A, F = shape
     adc = pkg.synth.cube_batch(F, S, C, A, cfg=11, n_targets=6)
     wr, wd = orc.hann_periodic(S), orc.hann_periodic(C)
     ref = orc.process_frames(adc, F, S, C, A, wr, wd, guard=guard, train=train, alpha=alpha, want=("P", "mask", "noise"))
@@ -143,7 +150,8 @@ def test_cfar_geometries(pkg, orc, guard, train, alpha):
 
 
 def _walk_form(F, Sp, Cp, sm_count):
-    """launch_cfar's rule for the default window: (range bins per strip, Doppler segments of 16 bins per CTA)"""
+    """launch_cfar's rule for the default window: (range bins per strip, Doppler segments of 16 bins per CTA, Sp the kernel
+    is specialised for or 0)"""
     cells, want = F * Sp * Cp, 8 * sm_count
     rt = 64
     if Sp % 128 == 0 and cells // (128 * 32) >= want:
@@ -153,7 +161,7 @@ def _walk_form(F, Sp, Cp, sm_count):
     nchunk = 2
     while nchunk < 8 and Cp % (32 * nchunk) == 0 and cells // (rt * 32 * nchunk) >= want:
         nchunk *= 2
-    return rt, nchunk
+    return rt, nchunk, (Sp if Sp in (256, 512, 1024) else 0)
 
 
 @pytest.fixture(scope="module")
@@ -162,26 +170,36 @@ def sm_count(pkg):
         return ctx.info.sm_count
 
 
-@pytest.mark.parametrize("variant", [1, 22, 42, 82, 23, 43, 83, 24, 44, 84])
-def test_cfar_kernel_forms_agree_with_oracle(pkg, orc, sm_count, variant):
+@pytest.mark.parametrize("form", WALK_FORMS, ids=lambda f: "tiled" if f is None else "rt%d-seg%d-spt%d" % f)
+def test_cfar_kernel_forms_agree_with_oracle(pkg, orc, sm_count, form):
     """Every form of K3 against the oracle's CFAR on the GPU's own power map: same mask away from threshold cells (the
-    clamped range edges included) and the noise estimate of every detection.  The forms are numbered as in the sweep
-    records (profiles/experiments/r1_cfar_walk_sweep.log): k + 10 * nchunk is the walk kernel with 64- / 128- / 256-bin
-    strips (k = 2 / 3 / 4) and Doppler segments of nchunk x 16 bins, reached through the batch size F for which
-    launch_cfar's rule picks it on this GPU (a few synthetic frames tiled to F); 1 is the tiled kernel, which serves every
-    window but the default one."""
-    if variant == 1:
+    clamped range edges included) and the noise estimate of every detection.  The walk kernel's forms are keyed as in
+    launch_cfar / run_cfar_walk: strips of 64 / 128 / 256 range bins, Doppler segments of nchunk x 16 bins per CTA, and
+    the Sp the kernel is specialised for (0: run-time Sp), reached through the shape and the batch size F for which
+    launch_cfar's rule picks it on this GPU (a few synthetic frames tiled to F); the tiled kernel serves every window but
+    the default one.  The kernel the batch launched is recorded and must be the one the form names, so a changed launcher
+    rule fails here instead of checking another form.  (Sweep records: profiles/experiments/r1_cfar_walk_sweep.log.)"""
+    if form is None:
         S, C, F, train = 256, 128, 2, (8, 5)
     else:
-        form = ({2: 64, 3: 128, 4: 256}[variant % 10], variant // 10)
-        S, C, F = next((S, C, F) for (S, C) in ((256, 128), (64, 256), (128, 256)) for F in range(1, 64 * sm_count)
-                       if _walk_form(F, S, C, sm_count) == form)
+        S, C, F = next((S, C, F) for (S, C) in ((256, 128), (64, 256), (128, 256), (512, 256), (1024, 64))
+                       for F in range(1, 64 * sm_count) if _walk_form(F, S, C, sm_count) == form)
         train = (8, 4)
     base = pkg.synth.cube_batch(3, S, C, 1, cfg=3, n_targets=6)
     adc = np.ascontiguousarray(base[np.arange(F) % 3])
+    import torch
+
     with pkg.RadarContext(S, C, 1, F, cfar_train=train) as ctx:
-        dets, overflow = ctx.process_host(adc, F)
+        # the device-resident entry point runs the whole batch as one: the host path uploads and processes it in chunks of
+        # 48 MB, which would take other forms for the frames of each chunk
+        adc_dev = torch.from_numpy(adc).cuda()
+        with launched_kernels() as names:
+            ctx.process_device(adc_dev, F)
+        dets, overflow = ctx.read_detections()
+        del adc_dev
         assert not overflow
+        cfar = sorted(k for k in names if k.startswith("cfar_"))
+        assert cfar == [cfar_form_name(form)], f"{S} x {C}, {F} frames launched {cfar}, not {cfar_form_name(form)}"
         frames = sorted({0, F // 2, F - 1})
         got = {f: (ctx.power_map(f), ctx.cfar_mask(f)) for f in frames}
     for f in frames:

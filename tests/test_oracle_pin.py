@@ -80,7 +80,10 @@ def test_legacy_edge_cases(orc):
     assert orc.lib().orc_find_abs_max(x.ctypes.data, 6553) == 100
 
 
-@pytest.mark.parametrize("S,C,A", [(64, 64, 2), (100, 128, 4), (128, 64, 12)])
+# after the first three: the ragged shapes test_gpu_kernel_forms.py checks the CUDA chain at against this oracle (S and C
+# zero-padded to the next power of two, up to 1000 x 998 -> 1024 x 1024)
+@pytest.mark.parametrize("S,C,A", [(64, 64, 2), (100, 128, 4), (128, 64, 12), (36, 34, 3), (60, 60, 2), (68, 66, 3),
+                                   (200, 130, 4), (300, 300, 2), (1000, 998, 2), (1000, 1000, 2)])
 def test_new_stages_against_numpy(orc, pkg, S, C, A):
     adc = pkg.synth.cube(3, S, C, A, cfg=5, n_targets=4)
     wr, wd = orc.hann_periodic(S), orc.hann_periodic(C)
@@ -94,18 +97,22 @@ def test_new_stages_against_numpy(orc, pkg, S, C, A):
     assert np.abs(out["rs"][0] - rs).max() <= 1e-12 * np.abs(rs).max()
     assert np.abs(out["dc"][0] - dc).max() <= 1e-12 * np.abs(dc).max()
     assert np.abs(out["P"][0] - P).max() <= 1e-12 * P.max()
-    # CFAR, brute force in numpy
+    # CFAR, brute force in numpy: every window cell added one by one (a shifted copy of the map per offset); range clamps
+    # (rows outside the map are zeros and are not counted), Doppler wraps
     Gr, Gd, Tr, Td, alpha = 2, 2, 8, 4, 15.0
     Wr, Wd = Gr + Tr, Gd + Td
-    noise = np.zeros_like(P)
-    for r in range(Sp):
-        rr = np.arange(max(0, r - Wr), min(Sp, r + Wr + 1))
-        gr = np.arange(max(0, r - Gr), min(Sp, r + Gr + 1))
-        for d in range(Cp):
-            dd = np.arange(d - Wd, d + Wd + 1) % Cp
-            gd = np.arange(d - Gd, d + Gd + 1) % Cp
-            tot = P[np.ix_(rr, dd)].sum() - P[np.ix_(gr, gd)].sum()
-            noise[r, d] = tot / (rr.size * dd.size - gr.size * gd.size)
+
+    def box(hr, hd):
+        Pz = np.pad(P, ((hr, hr), (0, 0)))
+        tot = np.zeros_like(P)
+        for i in range(2 * hr + 1):
+            for j in range(-hd, hd + 1):
+                tot += np.roll(Pz[i:i + Sp], -j, axis=1)
+        rows = np.minimum(np.arange(Sp) + hr, Sp - 1) - np.maximum(np.arange(Sp) - hr, 0) + 1
+        return tot, rows[:, None] * (2 * hd + 1)
+
+    (wt, wn), (gt, gn) = box(Wr, Wd), box(Gr, Gd)
+    noise = (wt - gt) / (wn - gn)
     thr = alpha * noise
     near = np.abs(P - thr) <= 1e-9 * thr
     assert np.allclose(out["noise"][0], noise, rtol=1e-6)
